@@ -28,6 +28,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(ROOT, "plonk-by-fingers_b200", "python"))
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (it may be read-only)
 
 METRIC = "plonk_by_hand_prove_plus_verify_throughput"
 UNIT = "proof+verify/s"
@@ -35,6 +36,8 @@ N_PER_GPU = 1 << 20
 SEED = 0xB200
 WORKLOAD = "batched prover+verifier: 2^20 D_fullpath witnesses of the pbh circuit per GPU per step, shared SRS (s=2, 7 points)"
 MASK64 = (1 << 64) - 1
+DUMP_ITEMS = 1 << 18                # --dump-outputs: items sampled from the per-item outputs
+DUMP_BITMAP_BYTES = 1 << 22         # --dump-outputs: leading bytes of the verdict bitmap kept
 
 
 def measured_peaks():
@@ -217,6 +220,29 @@ def roofline_entry(name, table_key, ms, items, bytes_per_item, peaks, instr):
     return ent
 
 
+def dump_outputs(out_dir, proof, status, result, bitmap, digest):
+    """Write what one step hands its caller as .npy files in float32 / float64 (under 64 MB in all), so that two builds
+    can be compared output for output: the proof planes, prover status and verdicts of a fixed, seeded sample of
+    DUMP_ITEMS items (their indices in item_index.npy), the verdict bitmap (its first DUMP_BITMAP_BYTES bytes when longer)
+    and the 64-bit proof digest as two exact 32-bit halves, low first."""
+    import numpy as np
+    n = status.numel()
+    if n > DUMP_ITEMS:
+        idx = np.sort(np.random.default_rng(SEED).choice(n, DUMP_ITEMS, replace=False))
+    else:
+        idx = np.arange(n)
+    d = int(digest.item()) & MASK64
+    arrays = {"item_index": idx.astype(np.float64),
+              "proof": proof.cpu().numpy()[:, idx].astype(np.float32),
+              "status": status.cpu().numpy()[idx].astype(np.float32),
+              "result": result.cpu().numpy()[idx].astype(np.float32),
+              "verdict_bitmap": bitmap[:DUMP_BITMAP_BYTES].cpu().numpy().astype(np.float32),
+              "proof_digest": np.array([d & 0xFFFFFFFF, d >> 32], dtype=np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -249,7 +275,12 @@ def main():
                     help="launch every prover from one stream (default: odd steps launch from a second prover stream, so prove(k+1) fills the SMs prove(k) leaves)")
     ap.add_argument("--no-overlap-verify", dest="overlap_verify", action="store_false",
                     help="keep verify(k) and prove(k+1) on one stream inside the graph (default: verify(k) runs on a second stream beside prove(k+1))")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (proofs, status, verdicts, bitmap, digest; rank 0) "
+                         "as DIR/<name>.npy in float32 / float64, per-item outputs as a fixed seeded sample")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -276,7 +307,7 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
 
     n = args.items
-    K = max(1, args.steps)
+    K = args.steps
     ctx = pbh_b200.Context(device=local, algo=args.algo)
     stream = ctx.torch_stream()
 
@@ -481,6 +512,12 @@ def main():
     launches = KERNELS_PER_STEP * K * reps
     value = n * world * K / (ms_total * 1e-3)
     last_set = (((K + ring - 1) // ring) - 1) % 2       # summary set written by the last cycle of a region
+    last_outputs = None
+    if args.dump_outputs and rank == 0:
+        # copied before the kernel timings below rewrite these buffers; written to DIR at the end
+        o = outs[(K - 1) % ring]
+        last_outputs = [t.clone() for t in (o["proof"], o["status"], o["result"], o["sets"][last_set]["bitmap"], o["sets"][last_set]["digest"])]
+        torch.cuda.synchronize()
 
     # ---- per-kernel durations for the roofline: each kernel alone, back to back over the ring, CUDA events on its stream
     def time_kernel(fn, reps_):
@@ -953,6 +990,8 @@ def main():
                      "accepted": best["accepted"], "equals_single_gpu": bool(np.array_equal(best["bitmap"], single_ref[0]) and best["total_digest"] == single_ref[1])}
     except Exception as e:   # pragma: no cover - reported, not fatal for the headline
         multi = {"error": f"{type(e).__name__}: {e}"}
+    if last_outputs is not None:
+        dump_outputs(args.dump_outputs, *last_outputs)
 
     line = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
