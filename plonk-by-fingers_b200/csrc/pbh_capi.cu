@@ -1763,7 +1763,8 @@ static int poly_unary_impl(pbh_ctx* ctx, size_t n, uint32_t len, const uint8_t* 
     d_out = stg.in<uint8_t>(nullptr, 0, n, pout, ce); CUDA_TRY(ctx, ce);
     ip = op = n;
   }
-  auto aligned = [&](size_t a) { return ((uintptr_t)d_in % a == 0) && ((uintptr_t)d_out % a == 0) && (ip % a == 0) && (op % a == 0); };
+  // eval writes one plane, so its output pitch (n, see pbh_poly_eval_batch) must not decide the access width
+  auto aligned = [&](size_t a) { return ((uintptr_t)d_in % a == 0) && ((uintptr_t)d_out % a == 0) && (ip % a == 0) && (pout == 1 || op % a == 0); };
   const int vec = aligned(16) ? 16 : (aligned(4) ? 4 : 0);
   poly_unary_kernel<OP><<<grid_for(ctx, vec ? (n + vec - 1) / vec : n, 8), kBlock, 0, ctx->compute>>>(n, len, d_in, ip, d_out, op, vec);
   SWEEP_FINISH(ctx);

@@ -311,7 +311,8 @@ def test_ntt4_intt4_exhaustive(gpu_ctx, oracle):
     ctx = gpu_ctx["table"]
     g = np.arange(17, dtype=np.uint8)
     v = np.stack(np.meshgrid(g, g, g, g, indexing="ij")).reshape(4, -1)
-    for arr in (v, v[:, :83521 - 3]):   # aligned (vector path) and ragged (byte tail)
+    # host planes are staged with pitch n: 83521 and 83518 take the byte loop, 83536 (padded with zeros) the 128-bit path
+    for arr in (v, v[:, :83521 - 3], np.pad(v, ((0, 0), (0, 83536 - 83521)))):
         arr = np.ascontiguousarray(arr)
         c = ctx.intt4_batch(arr)
         assert np.array_equal(c, oracle.intt4_batch(arr))
