@@ -40,8 +40,9 @@
 extern "C" {
 #endif
 
-/* 2: round 2 added entry points only (lanes, packed records, peer windows, multi-device, sweeps); every round-1 signature is unchanged */
-#define PBH_ABI_VERSION 2
+/* 2: round 2 added entry points only (lanes, packed records, peer windows, multi-device, sweeps); every round-1 signature is unchanged
+ * 3: entry points added (Fiat-Shamir over packed records), none changed */
+#define PBH_ABI_VERSION 3
 
 /* ---- errors (return values) ---------------------------------------------------------------- */
 typedef enum pbh_error {
@@ -271,6 +272,7 @@ int pbh_verify_fs_batch(pbh_ctx* ctx, size_t n, const uint8_t* proof, size_t pro
                         size_t chal_pitch, uint8_t* gt, size_t gt_pitch);
 int pbh_verify_fs_batch_dev(pbh_ctx* ctx, size_t n, const uint8_t* proof, size_t proof_pitch, uint8_t* result, uint8_t* chal_out,
                             size_t chal_pitch, uint8_t* gt, size_t gt_pitch);
+/* The same two calls over packed records: "Fiat-Shamir over packed records" below. */
 
 /* ---- record (array-of-structs) wire format — SURVEY.md §8(f) row 3 ---------------------------------------------
  * The reference has no serialisation (Proof only derives Debug, PartialEq: src/plonk.rs:61).  These 32-byte records let a
@@ -355,6 +357,41 @@ int pbh_unpack_witness_host(size_t n, const pbh_packed_witness* in, uint8_t* wit
 int pbh_pack_chal_u_host(size_t n, const uint8_t* chal, size_t chal_pitch, const uint8_t* u, uint32_t* out);
 int pbh_pack_proofs_host(size_t n, const uint8_t* proof, size_t proof_pitch, const uint8_t* status, pbh_packed_proof* out);
 int pbh_unpack_proofs_host(size_t n, const pbh_packed_proof* in, uint8_t* proof, size_t proof_pitch, uint8_t* status);
+
+/* ---- Fiat-Shamir over packed records: the two sections above combined ------------------------------------------------------
+ * A Fiat-Shamir prover takes no challenges and a Fiat-Shamir verifier takes only the proof, so the packed form of this family is
+ * 12 bytes up and 12 (+4) bytes down per proof, 12 bytes up and 1 byte down per verification:
+ *   pbh_packed_fs_witness  12 bytes: the 21 values wit[0..12) rand[0..9), each < 17, as base-17 digits, least significant first:
+ *                          values 0..6 in w[0], 7..13 in w[1], 14..20 in w[2] - word for word words 0..2 of pbh_packed_witness.
+ *                          Decoding is that of pbh_packed_witness: whatever lies above a word's seventh digit is folded into it
+ *                          and saturates at 255, so a word >= 17^7 decodes to a byte >= 17 and the item gets PBH_ST_BAD_ENCODING.
+ *   pbh_packed_proof       as above.
+ *   chal_u_out (nullable)  4 bytes per proof: the derived alpha beta gamma z v u as the chal_u word of pbh_verify_packed (six
+ *                          base-17 digits); zero where the status is not PBH_ST_OK, as chal_out of pbh_prove_fs_batch.  When it is
+ *                          null the prover skips the transcript step that derives u.
+ * PARITY UNPINNED BY THE REFERENCE, as both sections this one combines.  Definitions, bit for bit:
+ *   pbh_prove_fs_packed(in) = pack(pbh_prove_fs_batch(unpack(in))), with chal_u_out = pack_chal_u(chal_out);
+ *   pbh_verify_fs_packed(p) = pbh_verify_fs_batch(unpack(p)).
+ * A packed proof whose status code is not 0 decodes to the all-zero proof and is verified as such (PBH_VR_NOT_ON_CURVE).
+ * The kernels decode and encode in registers: there is no plane round trip and no extra launch.  Device record pointers must be
+ * 4-byte aligned.  The verifier always uploads and checks the buffer it is given. */
+typedef struct pbh_packed_fs_witness { uint32_t w[3]; } pbh_packed_fs_witness;
+/* HOST pointers (any memory; page-locked memory overlaps best), chunked over the staging buffers */
+int pbh_prove_fs_packed(pbh_ctx* ctx, size_t n, const pbh_packed_fs_witness* in, pbh_packed_proof* out, uint32_t* chal_u_out);
+int pbh_verify_fs_packed(pbh_ctx* ctx, size_t n, const pbh_packed_proof* proofs, uint8_t* result);
+/* the same on a lane, with the contract of pbh_prove_packed_async (pageable memory: waits for the context, then synchronous) */
+int pbh_prove_fs_packed_async(pbh_ctx* ctx, int lane, size_t n, const pbh_packed_fs_witness* in, pbh_packed_proof* out,
+                              uint32_t* chal_u_out);
+int pbh_verify_fs_packed_async(pbh_ctx* ctx, int lane, size_t n, const pbh_packed_proof* proofs, uint8_t* result);
+/* DEVICE pointers: only enqueued on the context's compute stream (may be captured into CUDA graphs) */
+int pbh_prove_fs_packed_dev(pbh_ctx* ctx, size_t n, const pbh_packed_fs_witness* in, pbh_packed_proof* out, uint32_t* chal_u_out);
+int pbh_verify_fs_packed_dev(pbh_ctx* ctx, size_t n, const pbh_packed_proof* proofs, uint8_t* result);
+/* host-side format conversion, as pbh_pack_witness_host / pbh_unpack_witness_host (PBH_ERR_BAD_ARGUMENT when a value is >= 17;
+ * null plane pointers are skipped by the unpack function) */
+int pbh_pack_fs_witness_host(size_t n, const uint8_t* wit, size_t wit_pitch, const uint8_t* rand, size_t rand_pitch,
+                             pbh_packed_fs_witness* out);
+int pbh_unpack_fs_witness_host(size_t n, const pbh_packed_fs_witness* in, uint8_t* wit, size_t wit_pitch, uint8_t* rand,
+                               size_t rand_pitch);
 
 /* ---- sweep kernels (the per-kernel configs of BASELINE.json), HOST or DEVICE pointers --------- */
 /* `on_device` != 0: pointers are device pointers, kernels are only enqueued.                      */

@@ -1616,6 +1616,180 @@ int pbh_unpack_proofs_host(size_t n, const pbh_packed_proof* in, uint8_t* proof,
   return PBH_OK;
 }
 
+// ---- Fiat-Shamir over packed records (include/pbh_b200.h) ---------------------------------------------------------------------
+static_assert(sizeof(pbh_packed_fs_witness) == 12, "packed Fiat-Shamir witnesses are 12 bytes");
+static int launch_prove_fs_packed(pbh_ctx* ctx, cudaStream_t st, size_t n, const pbh_packed_fs_witness* in, pbh_packed_proof* out,
+                                  uint32_t* chal_u_out) {
+  if (n == 0) return PBH_OK;
+  const int grid = grid_for(ctx, n, 2);
+  const FsSeed seed = fs_seed_of(ctx);
+  const bool special = ctx->pbh_circuit && ctx->specialise;
+  const uint32_t* i32 = reinterpret_cast<const uint32_t*>(in);
+  uint32_t* o32 = reinterpret_cast<uint32_t*>(out);
+  if (ctx->algo == PBH_ALGO_TABLE) {
+    if (!ctx->prover_fp32) prove_fs_packed_kernel<ALGO_TABLE, false, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, n, i32, o32, chal_u_out);
+    else if (special) prove_fs_packed_kernel<ALGO_TABLE, true, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, n, i32, o32, chal_u_out);
+    else prove_fs_packed_kernel<ALGO_TABLE, true, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, n, i32, o32, chal_u_out);
+  } else {
+    if (!ctx->prover_fp32) prove_fs_packed_kernel<ALGO_ARITH, false, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, n, i32, o32, chal_u_out);
+    else prove_fs_packed_kernel<ALGO_ARITH, true, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, n, i32, o32, chal_u_out);
+  }
+  ctx->launches++;
+  CUDA_TRY(ctx, cudaGetLastError());
+  return PBH_OK;
+}
+static int launch_verify_fs_packed(pbh_ctx* ctx, cudaStream_t st, size_t n, const pbh_packed_proof* proofs, uint8_t* result) {
+  if (n == 0) return PBH_OK;
+  const int grid = grid_for(ctx, n, 2);
+  const FsSeed seed = fs_seed_of(ctx);
+  const uint32_t* p32 = reinterpret_cast<const uint32_t*>(proofs);
+  if (ctx->algo == PBH_ALGO_TABLE)
+    verify_fs_packed_kernel<ALGO_TABLE><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, ctx->verifier_fp32 != 0, seed, ctx->d_tables, n, p32, result);
+  else verify_fs_packed_kernel<ALGO_ARITH><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, false, seed, ctx->d_tables, n, p32, result);
+  ctx->launches++;
+  CUDA_TRY(ctx, cudaGetLastError());
+  return PBH_OK;
+}
+static bool aligned4(const void* p) { return ((uintptr_t)p % 4) == 0; }
+
+int pbh_prove_fs_packed_dev(pbh_ctx* ctx, size_t n, const pbh_packed_fs_witness* in, pbh_packed_proof* out, uint32_t* chal_u_out) {
+  CTX_CHECK(ctx);
+  if (n == 0) return PBH_OK;
+  if (!in || !out) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
+  if (!aligned4(in) || !aligned4(out) || !aligned4(chal_u_out)) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "packed records must be 4-byte aligned");
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  return launch_prove_fs_packed(ctx, ctx->compute, n, in, out, chal_u_out);
+}
+int pbh_verify_fs_packed_dev(pbh_ctx* ctx, size_t n, const pbh_packed_proof* proofs, uint8_t* result) {
+  CTX_CHECK(ctx);
+  if (n == 0) return PBH_OK;
+  if (!proofs || !result) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
+  if (!aligned4(proofs)) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "packed proofs must be 4-byte aligned");
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  return launch_verify_fs_packed(ctx, ctx->compute, n, proofs, result);
+}
+
+// One chunk (or one whole lane batch) on stream st, staged in `base` (rows of C bytes): the prover's records in rows 64..75, its
+// proofs in 80..91 and challenge words in 92..95; the verifier's proofs in 96..107 and results in row 108.  Prover and verifier
+// rows are disjoint, so a verify enqueued on a lane behind a prove never overwrites rows that prove still has to download.
+static_assert(64 + sizeof(pbh_packed_fs_witness) <= 80 && 80 + sizeof(pbh_packed_proof) + 4 <= 96 && 96 + sizeof(pbh_packed_proof) + 1 <= kStagePlanes,
+              "packed Fiat-Shamir bodies: prover rows 64..95, verifier rows 96..108");
+static int fs_packed_prove_body(pbh_ctx* ctx, cudaStream_t st, uint8_t* base, size_t C, size_t m, const pbh_packed_fs_witness* in,
+                                pbh_packed_proof* out, uint32_t* chal_u_out) {
+  pbh_packed_fs_witness* d_in = reinterpret_cast<pbh_packed_fs_witness*>(base + 64 * C);
+  pbh_packed_proof* d_out = reinterpret_cast<pbh_packed_proof*>(base + 80 * C);
+  uint32_t* d_cu = reinterpret_cast<uint32_t*>(base + 92 * C);
+  PBH_TRY(stage_h2d(ctx, base, st, d_in, 0, in, 0, m * sizeof(pbh_packed_fs_witness), 1));
+  PBH_TRY(launch_prove_fs_packed(ctx, st, m, d_in, d_out, chal_u_out ? d_cu : nullptr));
+  PBH_TRY(stage_d2h(ctx, base, st, out, 0, d_out, 0, m * sizeof(pbh_packed_proof), 1));
+  if (chal_u_out) PBH_TRY(stage_d2h(ctx, base, st, chal_u_out, 0, d_cu, 0, m * sizeof(uint32_t), 1));
+  return PBH_OK;
+}
+static int fs_packed_verify_body(pbh_ctx* ctx, cudaStream_t st, uint8_t* base, size_t C, size_t m, const pbh_packed_proof* proofs,
+                                 uint8_t* result) {
+  pbh_packed_proof* d_prf = reinterpret_cast<pbh_packed_proof*>(base + 96 * C);
+  uint8_t* d_res = base + 108 * C;
+  PBH_TRY(stage_h2d(ctx, base, st, d_prf, 0, proofs, 0, m * sizeof(pbh_packed_proof), 1));
+  PBH_TRY(launch_verify_fs_packed(ctx, st, m, d_prf, d_res));
+  PBH_TRY(stage_d2h(ctx, base, st, result, 0, d_res, 0, m, 1));
+  return PBH_OK;
+}
+
+int pbh_prove_fs_packed(pbh_ctx* ctx, size_t n, const pbh_packed_fs_witness* in, pbh_packed_proof* out, uint32_t* chal_u_out) {
+  CTX_CHECK(ctx);
+  if (n == 0) return PBH_OK;
+  if (!in || !out) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  return for_each_chunk(ctx, n, [&](size_t lo, size_t m, size_t C, uint8_t* base, cudaStream_t st) -> int {
+    return fs_packed_prove_body(ctx, st, base, C, m, in + lo, out + lo, chal_u_out ? chal_u_out + lo : nullptr);
+  });
+}
+int pbh_verify_fs_packed(pbh_ctx* ctx, size_t n, const pbh_packed_proof* proofs, uint8_t* result) {
+  CTX_CHECK(ctx);
+  if (n == 0) return PBH_OK;
+  if (!proofs || !result) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  return for_each_chunk(ctx, n, [&](size_t lo, size_t m, size_t C, uint8_t* base, cudaStream_t st) -> int {
+    return fs_packed_verify_body(ctx, st, base, C, m, proofs + lo, result + lo);
+  });
+}
+// A lane call that fails after enqueueing copies waits for them: the caller may release its buffers once the call has returned.
+static int lane_settle(pbh_ctx* ctx, cudaStream_t st, int rc) {
+  if (rc != PBH_OK) {
+    const std::string keep = ctx->last_error;
+    cudaStreamSynchronize(st);
+    cudaGetLastError();
+    ctx->last_error = keep;
+  }
+  return rc;
+}
+int pbh_prove_fs_packed_async(pbh_ctx* ctx, int lane, size_t n, const pbh_packed_fs_witness* in, pbh_packed_proof* out, uint32_t* chal_u_out) {
+  CTX_CHECK(ctx);
+  cudaStream_t st;
+  int rc = lane_stream(ctx, lane, &st);
+  if (rc) return rc;
+  ctx->resident_host[lane] = nullptr;
+  if (n == 0) return PBH_OK;
+  if (!in || !out) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  if (n <= kLaneMaxItems && host_pinned(reinterpret_cast<const uint8_t*>(in)) && host_pinned(reinterpret_cast<const uint8_t*>(out)) &&
+      (!chal_u_out || host_pinned(reinterpret_cast<const uint8_t*>(chal_u_out)))) {
+    const size_t C = (n + kTile - 1) / kTile * kTile;
+    rc = ensure_lane(ctx, lane, kStagePlanes * C);
+    if (rc) return rc;
+    return lane_settle(ctx, st, fs_packed_prove_body(ctx, st, ctx->lane_buf[lane], C, n, in, out, chal_u_out));
+  }
+  rc = pbh_ctx_sync(ctx);
+  if (rc) return rc;
+  return pbh_prove_fs_packed(ctx, n, in, out, chal_u_out);
+}
+// No resident-proof shortcut here (PBH_OPT_PROOF_RESIDENT): the verifier uploads the buffer it is handed, whatever ran before.
+int pbh_verify_fs_packed_async(pbh_ctx* ctx, int lane, size_t n, const pbh_packed_proof* proofs, uint8_t* result) {
+  CTX_CHECK(ctx);
+  cudaStream_t st;
+  int rc = lane_stream(ctx, lane, &st);
+  if (rc) return rc;
+  ctx->resident_host[lane] = nullptr;
+  if (n == 0) return PBH_OK;
+  if (!proofs || !result) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  if (n <= kLaneMaxItems && host_pinned(reinterpret_cast<const uint8_t*>(proofs)) && host_pinned(result)) {
+    const size_t C = (n + kTile - 1) / kTile * kTile;
+    rc = ensure_lane(ctx, lane, kStagePlanes * C);
+    if (rc) return rc;
+    return lane_settle(ctx, st, fs_packed_verify_body(ctx, st, ctx->lane_buf[lane], C, n, proofs, result));
+  }
+  rc = pbh_ctx_sync(ctx);
+  if (rc) return rc;
+  return pbh_verify_fs_packed(ctx, n, proofs, result);
+}
+
+int pbh_pack_fs_witness_host(size_t n, const uint8_t* wit, size_t wit_pitch, const uint8_t* rnd, size_t rand_pitch, pbh_packed_fs_witness* out) {
+  if (n == 0) return PBH_OK;
+  if (!wit || !rnd || !out || wit_pitch < n || rand_pitch < n) return PBH_ERR_BAD_ARGUMENT;
+  bool ok = true;
+  for (size_t i = 0; i < n; i++) {
+    uint8_t v[27] = {0};   // chal and u stay zero: word 3 of the full witness is not part of this record
+    for (int k = 0; k < 12; k++) v[k] = wit[k * wit_pitch + i];
+    for (int k = 0; k < 9; k++) v[12 + k] = rnd[k * rand_pitch + i];
+    uint32_t w[4];
+    ok = pack_witness_item(v, w) && ok;
+    for (int j = 0; j < 3; j++) out[i].w[j] = w[j];
+  }
+  return ok ? PBH_OK : PBH_ERR_BAD_ARGUMENT;
+}
+int pbh_unpack_fs_witness_host(size_t n, const pbh_packed_fs_witness* in, uint8_t* wit, size_t wit_pitch, uint8_t* rnd, size_t rand_pitch) {
+  if (n == 0) return PBH_OK;
+  if (!in || (wit && wit_pitch < n) || (rnd && rand_pitch < n)) return PBH_ERR_BAD_ARGUMENT;
+  for (size_t i = 0; i < n; i++) {
+    uint8_t v[21];
+    for (int j = 0; j < 3; j++) digits17<7>(in[i].w[j], v + 7 * j);
+    if (wit) for (int k = 0; k < 12; k++) wit[k * wit_pitch + i] = v[k];
+    if (rnd) for (int k = 0; k < 9; k++) rnd[k * rand_pitch + i] = v[12 + k];
+  }
+  return PBH_OK;
+}
+
 // ---- sweep entry points ---------------------------------------------------------------------------------
 // Host-pointer mode stages whole planes through a temporary device allocation (these are per-kernel test and
 // benchmark entry points; the hot host-pointer path is pbh_prove_batch / pbh_verify_batch above).

@@ -14,6 +14,7 @@
 #include "pbh_verify.cuh"
 #include "pbh_prove_f32.cuh"
 #include "pbh_tma.cuh"
+#include "pbh_packed.cuh"
 
 namespace pbh {
 
@@ -453,6 +454,94 @@ __global__ void __launch_bounds__(256, 2) verify_fs_kernel(const Consts K, const
 #pragma unroll
       for (int k = 0; k < 6; k++) F.chal_out[(size_t)k * F.chal_pitch + i] = (uint8_t)derived[k];
     }
+  }
+}
+
+// ---- Fiat-Shamir over packed records (include/pbh_b200.h): the codec of pbh_packed.cuh runs in registers around the same per-item
+// routines, so no plane ever reaches memory.  12 bytes in and 12 (+4) out per proof, 12 in and 1 out per verification; records are
+// read and written as three 32-bit words per thread (a warp touches 384 contiguous bytes), the kernels stay ALU-bound.
+template <int ALGO, bool FP32, bool PBH_CIRCUIT>
+__global__ void __launch_bounds__(256, 2) prove_fs_packed_kernel(const Consts K, const ConstsF KF, const FsSeed seed, const Tables* __restrict__ gT,
+                                                                  size_t n, const uint32_t* __restrict__ in, uint32_t* __restrict__ out,
+                                                                  uint32_t* __restrict__ chal_u_out) {
+  __shared__ Tables sT;
+  __shared__ PackedTables sP;
+  stage_packed_tables(&sP);
+  stage_tables(sT, gT);
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+    uint8_t v[21];
+    digits17<7>(in[3 * i], v);
+    digits17<7>(in[3 * i + 1], v + 7);
+    digits17<7>(in[3 * i + 2], v + 14);
+    uint32_t w[12], r[9];
+    bool bad = false;
+#pragma unroll
+    for (int k = 0; k < 12; k++) { w[k] = v[k]; bad = bad || w[k] >= 17u; }
+#pragma unroll
+    for (int k = 0; k < 9; k++) { r[k] = v[12 + k]; bad = bad || r[k] >= 17u; }
+    if (bad) {
+#pragma unroll
+      for (int k = 0; k < 12; k++) w[k] = 0;
+#pragma unroll
+      for (int k = 0; k < 9; k++) r[k] = 0;
+    }
+    ProofRegs P;
+    uint32_t derived[6];
+    uint32_t status = prove_item_fs<ALGO, FP32, PBH_CIRCUIT>(w, r, seed.w, K, KF, sT, P, derived, chal_u_out != nullptr);
+    if (bad) status = PBH_ST_BAD_ENCODING;
+    // the 27 bytes store_proof would write
+    const bool ok = status == 0u;
+    uint8_t p[27];
+    uint32_t inf_lo = 0, inf_hi = 0;
+#pragma unroll
+    for (int k = 0; k < 9; k++) {
+      const uint32_t pw = ok ? P.pt[k] : 0u;
+      p[2 * k] = (uint8_t)(pw & 0xFF);
+      p[2 * k + 1] = (uint8_t)((pw >> 8) & 0xFF);
+      const uint32_t inf = (pw >> 16) & 1u;
+      if (k < 8) inf_lo |= inf << k; else inf_hi |= inf;
+    }
+    p[PBH_PROOF_INF_PLANE] = (uint8_t)inf_lo;
+    p[PBH_PROOF_INF_PLANE + 1] = (uint8_t)inf_hi;
+#pragma unroll
+    for (int k = 0; k < 7; k++) p[PBH_PROOF_EVAL_PLANE + k] = (uint8_t)(ok ? P.ev[k] : 0u);
+    uint32_t o[3];
+    pack_proof_item(sP, p, (uint8_t)status, o);
+    out[3 * i] = o[0];
+    out[3 * i + 1] = o[1];
+    out[3 * i + 2] = o[2];
+    if (chal_u_out) {
+      // digits alpha beta gamma z v u, least significant first (pack_chal_u); every derived value is < 17
+      uint32_t cu = 0;
+#pragma unroll
+      for (int k = 5; k >= 0; k--) cu = cu * 17u + derived[k];
+      chal_u_out[i] = ok ? cu : 0u;
+    }
+  }
+}
+
+// A packed proof whose status code is not 0 decodes to the all-zero proof and goes through verify_one_fs like any other.
+template <int ALGO>
+__global__ void __launch_bounds__(256, 2) verify_fs_packed_kernel(const Consts K, const ConstsF KF, const bool fp32, const FsSeed seed,
+                                                                   const Tables* __restrict__ gT, size_t n, const uint32_t* __restrict__ proofs,
+                                                                   uint8_t* __restrict__ result) {
+  __shared__ Tables sT;
+  __shared__ PackedTables sP;
+  stage_packed_tables(&sP);
+  stage_tables(sT, gT);
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+    const uint32_t wd[3] = {proofs[3 * i], proofs[3 * i + 1], proofs[3 * i + 2]};
+    uint8_t p[27], st;
+    unpack_proof_item(sP, wd, p, &st);
+    uint32_t px[9], py[9], ev[7];
+#pragma unroll
+    for (int k = 0; k < 9; k++) { px[k] = p[2 * k]; py[k] = p[2 * k + 1]; }
+    const uint32_t infbits = (uint32_t)p[PBH_PROOF_INF_PLANE] | ((uint32_t)p[PBH_PROOF_INF_PLANE + 1] << 8);
+#pragma unroll
+    for (int k = 0; k < 7; k++) ev[k] = p[PBH_PROOF_EVAL_PLANE + k];
+    GT e1, e2;
+    uint32_t derived[6];
+    result[i] = (uint8_t)verify_one_fs<ALGO>(px, py, infbits, ev, seed.w, K, sT, e1, e2, fp32 ? &KF : nullptr, derived);
   }
 }
 

@@ -53,7 +53,9 @@ pbh_multi_set_algo pbh_multi_prove_batch pbh_multi_verify_batch pbh_multi_prove_
 pbh_gt_mul_batch pbh_gt_pow600_batch pbh_poly_divrem_batch pbh_poly_addsub_ragged_batch
 pbh_prove_packed pbh_verify_packed pbh_prove_packed_async pbh_verify_packed_async pbh_prove_verify_packed pbh_unpack_witness_dev
 pbh_pack_proof_dev pbh_unpack_proof_dev pbh_pack_witness_host pbh_unpack_witness_host pbh_pack_chal_u_host pbh_pack_proofs_host
-pbh_unpack_proofs_host pbh_window_create pbh_window_attach pbh_window_attach_ptrs pbh_window_share pbh_window_destroy pbh_multi_prove_packed pbh_multi_verify_packed pbh_prove_verify_packed_async pbh_host_alloc_input""".split()
+pbh_unpack_proofs_host pbh_window_create pbh_window_attach pbh_window_attach_ptrs pbh_window_share pbh_window_destroy pbh_multi_prove_packed pbh_multi_verify_packed pbh_prove_verify_packed_async pbh_host_alloc_input
+pbh_prove_fs_packed pbh_verify_fs_packed pbh_prove_fs_packed_async pbh_verify_fs_packed_async pbh_prove_fs_packed_dev pbh_verify_fs_packed_dev
+pbh_pack_fs_witness_host pbh_unpack_fs_witness_host""".split()
 
 
 # 32-byte records of include/pbh_b200.h
@@ -110,6 +112,8 @@ class Circuit(C.Structure):
 # packed records of include/pbh_b200.h ("packed wire format"): 16-byte prover inputs, 12-byte proofs, 4-byte challenge words
 PACKED_WITNESS = np.dtype([("w", "<u4", (4,))])
 PACKED_PROOF = np.dtype([("points_lo", "<u4"), ("points_hi", "<u4"), ("evals_status", "<u4")])
+# Fiat-Shamir prover input: wit + rand only, words 0..2 of PACKED_WITNESS
+PACKED_FS_WITNESS = np.dtype([("w", "<u4", (3,))])
 ST_UNREPRESENTABLE = 33
 
 
@@ -149,6 +153,33 @@ def unpack_witness(packed):
     if rc != 0:
         raise PbhError(f"pbh_unpack_witness_host: {ERR.get(rc, rc)}")
     return wit, rand, chal, u[0]
+
+
+def pack_fs_witness(wit, rand):
+    """Byte planes (host) -> PACKED_FS_WITNESS array (pbh_pack_fs_witness_host, a CPU format conversion)."""
+    lib = load_library()
+    W = _host_u8(wit, 12, "wit"); n = W.shape[1]
+    R = _host_u8(rand, 9, "rand")
+    if R.shape[1] != n:
+        raise PbhError("wit and rand must have the same number of items")
+    out = np.zeros(n, dtype=PACKED_FS_WITNESS)
+    rc = lib.pbh_pack_fs_witness_host(C.c_size_t(n), C.c_void_p(W.ctypes.data), C.c_size_t(n), C.c_void_p(R.ctypes.data), C.c_size_t(n),
+                                      C.c_void_p(out.ctypes.data))
+    if rc != 0:
+        raise PbhError(f"pbh_pack_fs_witness_host: {ERR.get(rc, rc)} (a value >= 17 has no packed form)")
+    return out
+
+
+def unpack_fs_witness(packed):
+    """PACKED_FS_WITNESS array -> (wit, rand) byte planes."""
+    lib = load_library()
+    pk = np.ascontiguousarray(packed, dtype=PACKED_FS_WITNESS); n = pk.shape[0]
+    wit, rand = np.zeros((12, n), np.uint8), np.zeros((9, n), np.uint8)
+    rc = lib.pbh_unpack_fs_witness_host(C.c_size_t(n), C.c_void_p(pk.ctypes.data), C.c_void_p(wit.ctypes.data), C.c_size_t(n),
+                                        C.c_void_p(rand.ctypes.data), C.c_size_t(n))
+    if rc != 0:
+        raise PbhError(f"pbh_unpack_fs_witness_host: {ERR.get(rc, rc)}")
+    return wit, rand
 
 
 def pack_chal_u(chal, u):
@@ -666,6 +697,80 @@ class Context:
             raise PbhError("packed_in, out and result must have the same length")
         self._check(self.lib.pbh_prove_verify_packed_async(self.h, int(lane), C.c_size_t(pin.shape[0]), C.c_void_p(pin.ctypes.data),
                                                            C.c_void_p(o.ctypes.data), C.c_void_p(res.ctypes.data)), "pbh_prove_verify_packed_async")
+
+    # ---- Fiat-Shamir over packed records (12-byte prover inputs, 12-byte proofs, optional 4-byte challenge words) ----
+    # numpy arrays select the host-pointer calls; CUDA tensors (contiguous, any dtype, viewed as bytes) select the `_dev` calls,
+    # whose outputs are uint8 tensors of 12 (proofs) / 4 (challenge words) / 1 (results) bytes per item.
+    def _dev_records(self, t, itemsize, name, n=None):
+        if not t.is_cuda or not t.is_contiguous():
+            raise PbhError(f"{name}: device records must be a contiguous CUDA tensor")
+        nbytes = t.numel() * t.element_size()
+        if nbytes % itemsize or (n is not None and nbytes != n * itemsize):
+            raise PbhError(f"{name}: expected {'n' if n is None else n} records of {itemsize} bytes, got {nbytes} bytes")
+        return t, nbytes // itemsize
+
+    def _dev_bytes(self, n, itemsize):
+        import torch
+        return torch.empty((n * itemsize,), dtype=torch.uint8, device=torch.device("cuda", self.device))
+
+    def prove_fs_packed(self, packed_in, out=None, chal_u=None, want_chal_u=True):
+        """PACKED_FS_WITNESS records -> PACKED_PROOF records [, challenge words alpha beta gamma z v u]:
+        pack(pbh_prove_fs_batch(unpack(in))).  numpy = host call, torch.cuda = device call."""
+        if _is_torch(packed_in):
+            pin, n = self._dev_records(packed_in, 12, "packed_in")
+            out = self._dev_bytes(n, 12) if out is None else self._dev_records(out, 12, "out", n)[0]
+            if want_chal_u or chal_u is not None:
+                chal_u = self._dev_bytes(n, 4) if chal_u is None else self._dev_records(chal_u, 4, "chal_u", n)[0]
+            cur = self._dev_begin()
+            rc = self.lib.pbh_prove_fs_packed_dev(self.h, C.c_size_t(n), C.c_void_p(pin.data_ptr()), C.c_void_p(out.data_ptr()),
+                                                  C.c_void_p(chal_u.data_ptr() if chal_u is not None else None))
+            self._dev_end(cur)
+            self._check(rc, "pbh_prove_fs_packed_dev")
+        else:
+            pin = self._packed(packed_in, PACKED_FS_WITNESS, "packed_in"); n = pin.shape[0]
+            out = np.zeros(n, dtype=PACKED_PROOF) if out is None else self._packed(out, PACKED_PROOF, "out", True)
+            if want_chal_u or chal_u is not None:
+                chal_u = np.zeros(n, dtype="<u4") if chal_u is None else self._packed(chal_u, np.dtype("<u4"), "chal_u", True)
+            if out.shape[0] != n or (chal_u is not None and chal_u.shape[0] != n):
+                raise PbhError("packed_in, out and chal_u must have the same length")
+            self._check(self.lib.pbh_prove_fs_packed(self.h, C.c_size_t(n), C.c_void_p(pin.ctypes.data), C.c_void_p(out.ctypes.data),
+                                                     C.c_void_p(chal_u.ctypes.data if chal_u is not None else None)), "pbh_prove_fs_packed")
+        return (out, chal_u) if chal_u is not None else out
+
+    def verify_fs_packed(self, proofs, result=None):
+        """PACKED_PROOF records -> result bytes (PBH_VR_*): pbh_verify_fs_batch(unpack(proofs)).  numpy = host, torch.cuda = device."""
+        if _is_torch(proofs):
+            prf, n = self._dev_records(proofs, 12, "proofs")
+            result = self._dev_bytes(n, 1) if result is None else self._dev_records(result, 1, "result", n)[0]
+            cur = self._dev_begin()
+            rc = self.lib.pbh_verify_fs_packed_dev(self.h, C.c_size_t(n), C.c_void_p(prf.data_ptr()), C.c_void_p(result.data_ptr()))
+            self._dev_end(cur)
+            self._check(rc, "pbh_verify_fs_packed_dev")
+            return result
+        prf = self._packed(proofs, PACKED_PROOF, "proofs"); n = prf.shape[0]
+        res = np.zeros(n, dtype=np.uint8) if result is None else self._packed(result, np.dtype(np.uint8), "result", True)
+        if res.shape[0] != n:
+            raise PbhError("proofs and result must have the same length")
+        self._check(self.lib.pbh_verify_fs_packed(self.h, C.c_size_t(n), C.c_void_p(prf.ctypes.data), C.c_void_p(res.ctypes.data)),
+                    "pbh_verify_fs_packed")
+        return res
+
+    def prove_fs_packed_async(self, lane, packed_in, out, chal_u=None):
+        """Enqueue pbh_prove_fs_packed on `lane`; the arrays must stay alive and untouched until lane_sync(lane)."""
+        pin = self._packed(packed_in, PACKED_FS_WITNESS, "packed_in"); o = self._packed(out, PACKED_PROOF, "out", True)
+        cu = self._packed(chal_u, np.dtype("<u4"), "chal_u", True) if chal_u is not None else None
+        if o.shape[0] != pin.shape[0] or (cu is not None and cu.shape[0] != pin.shape[0]):
+            raise PbhError("packed_in, out and chal_u must have the same length")
+        self._check(self.lib.pbh_prove_fs_packed_async(self.h, int(lane), C.c_size_t(pin.shape[0]), C.c_void_p(pin.ctypes.data),
+                                                       C.c_void_p(o.ctypes.data), C.c_void_p(cu.ctypes.data if cu is not None else None)),
+                    "pbh_prove_fs_packed_async")
+
+    def verify_fs_packed_async(self, lane, proofs, result):
+        prf = self._packed(proofs, PACKED_PROOF, "proofs"); res = self._packed(result, np.dtype(np.uint8), "result", True)
+        if res.shape[0] != prf.shape[0]:
+            raise PbhError("proofs and result must have the same length")
+        self._check(self.lib.pbh_verify_fs_packed_async(self.h, int(lane), C.c_size_t(prf.shape[0]), C.c_void_p(prf.ctypes.data),
+                                                        C.c_void_p(res.ctypes.data)), "pbh_verify_fs_packed_async")
 
     def host_alloc_as(self, n, dtype, write_combined=False):
         """host_alloc viewed as n records of `dtype` (page-locked memory for the packed lane calls)."""

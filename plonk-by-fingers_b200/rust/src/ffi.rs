@@ -101,6 +101,19 @@ extern "C" {
     pub fn pbh_pack_chal_u_host(n: usize, chal: *const u8, chal_pitch: usize, u: *const u8, out: *mut u32) -> c_int;
     pub fn pbh_pack_proofs_host(n: usize, proof: *const u8, proof_pitch: usize, status: *const u8, out: *mut PackedProof) -> c_int;
     pub fn pbh_unpack_proofs_host(n: usize, input: *const PackedProof, proof: *mut u8, proof_pitch: usize, status: *mut u8) -> c_int;
+    // Fiat-Shamir over packed records: 12-byte prover inputs (wit + rand), 12-byte proofs, optional 4-byte derived challenge words
+    pub fn pbh_prove_fs_packed(ctx: *mut pbh_ctx, n: usize, input: *const PackedFsWitness, out: *mut PackedProof, chal_u_out: *mut u32) -> c_int;
+    pub fn pbh_verify_fs_packed(ctx: *mut pbh_ctx, n: usize, proofs: *const PackedProof, result: *mut u8) -> c_int;
+    pub fn pbh_prove_fs_packed_async(ctx: *mut pbh_ctx, lane: c_int, n: usize, input: *const PackedFsWitness, out: *mut PackedProof,
+                                     chal_u_out: *mut u32) -> c_int;
+    pub fn pbh_verify_fs_packed_async(ctx: *mut pbh_ctx, lane: c_int, n: usize, proofs: *const PackedProof, result: *mut u8) -> c_int;
+    pub fn pbh_prove_fs_packed_dev(ctx: *mut pbh_ctx, n: usize, input: *const PackedFsWitness, out: *mut PackedProof,
+                                   chal_u_out: *mut u32) -> c_int;
+    pub fn pbh_verify_fs_packed_dev(ctx: *mut pbh_ctx, n: usize, proofs: *const PackedProof, result: *mut u8) -> c_int;
+    pub fn pbh_pack_fs_witness_host(n: usize, wit: *const u8, wit_pitch: usize, rand: *const u8, rand_pitch: usize,
+                                    out: *mut PackedFsWitness) -> c_int;
+    pub fn pbh_unpack_fs_witness_host(n: usize, input: *const PackedFsWitness, wit: *mut u8, wit_pitch: usize, rand: *mut u8,
+                                      rand_pitch: usize) -> c_int;
     // batched equivalents of the crate's value-type operations (a selection; the header has them all)
     pub fn pbh_kzg_commit_batch(ctx: *mut pbh_ctx, n: usize, coeffs: *const u8, in_pitch: usize, out: *mut u8, out_pitch: usize,
                                 on_device: c_int) -> c_int;                       // SRS::eval_at_s
@@ -150,3 +163,6 @@ pub struct PackedWitness { pub w: [u32; 4] }
 #[repr(C)]
 #[derive(Clone, Copy, Default, PartialEq, Eq, Debug)]
 pub struct PackedProof { pub points_lo: u32, pub points_hi: u32, pub evals_status: u32 }
+#[repr(C)]
+#[derive(Clone, Copy, Default, PartialEq, Eq, Debug)]
+pub struct PackedFsWitness { pub w: [u32; 3] }
