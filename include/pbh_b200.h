@@ -41,8 +41,9 @@ extern "C" {
 #endif
 
 /* 2: round 2 added entry points only (lanes, packed records, peer windows, multi-device, sweeps); every round-1 signature is unchanged
- * 3: entry points added (Fiat-Shamir over packed records), none changed */
-#define PBH_ABI_VERSION 3
+ * 3: entry points added (Fiat-Shamir over packed records), none changed
+ * 4: entry points added (Fiat-Shamir shard summaries and multi-device calls), none changed */
+#define PBH_ABI_VERSION 4
 
 /* ---- errors (return values) ---------------------------------------------------------------- */
 typedef enum pbh_error {
@@ -496,13 +497,22 @@ int pbh_prove_digest_batch_dev(pbh_ctx* ctx, size_t n, const uint8_t* wit, size_
                                uint8_t* status, uint64_t first_index, uint64_t* digest);
 int pbh_verify_bitmap_batch_dev(pbh_ctx* ctx, size_t n, const uint8_t* proof, size_t proof_pitch, const uint8_t* chal,
                                 size_t chal_pitch, const uint8_t* u, uint8_t* result, uint8_t* bitmap);
+/* The same for the Fiat-Shamir calls: pbh_prove_fs_batch_dev followed by pbh_digest_dev(27 proof planes, first_index), and
+ * pbh_verify_fs_batch_dev followed by pbh_pack_verdicts_dev(result).  chal_out (nullable) as in pbh_prove_fs_batch_dev.  The
+ * FP32 provers add the digest in the kernel; with PBH_OPT_PROVER_FP32 = 0 the digest kernel runs after the prover.  A bitmap
+ * that is not 4-byte aligned is packed by a second kernel.  Both take part in peer windows like the two calls above. */
+int pbh_prove_fs_digest_batch_dev(pbh_ctx* ctx, size_t n, const uint8_t* wit, size_t wit_pitch, const uint8_t* rand,
+                                  size_t rand_pitch, uint8_t* proof, size_t proof_pitch, uint8_t* status, uint8_t* chal_out,
+                                  size_t chal_pitch, uint64_t first_index, uint64_t* digest);
+int pbh_verify_fs_bitmap_batch_dev(pbh_ctx* ctx, size_t n, const uint8_t* proof, size_t proof_pitch, uint8_t* result,
+                                   uint8_t* bitmap);
 
 /* ---- peer windows: the gather of the shard summaries as plain stores over NVLink ----------------------------------------
  * The only exchange of the sharded path is that every device ends up with every shard's verdict bitmap and proof digest
  * (SURVEY.md 8e).  A collective after the kernels costs a rendezvous per call; a peer window removes it: every rank owns a
  * device buffer of world x bytes_per_rank bytes, rank r's region being bytes [r * bytes_per_rank, (r + 1) * bytes_per_rank)
- * of EVERY rank's buffer.  When the `digest` of pbh_prove_digest_batch_dev or the `bitmap` of pbh_verify_bitmap_batch_dev
- * points into the calling rank's own region, the kernel that produces the summary also stores it at the same offset of every
+ * of EVERY rank's buffer.  When the `digest` of pbh_prove_digest_batch_dev / pbh_prove_fs_digest_batch_dev or the `bitmap` of
+ * pbh_verify_bitmap_batch_dev / pbh_verify_fs_bitmap_batch_dev points into the calling rank's own region, the kernel that produces the summary also stores it at the same offset of every
  * peer's buffer - the verifier per 256-item tile (one 32-byte store per peer), the prover's last block its 8-byte digest -
  * through peer-mapped device memory (NVLink / NVSwitch), so the all-gather has happened when the kernels have finished and
  * costs neither a launch nor a rendezvous.  A consumer on another rank must be ordered after the producing rank's stream
@@ -555,6 +565,20 @@ int pbh_multi_verify_packed(pbh_multi* m, size_t n, const pbh_packed_proof* proo
 int pbh_multi_prove_verify_sharded(pbh_multi* m, uint64_t n_total, uint64_t first_index, uint64_t seed, int dist,
                                    uint8_t* bitmap_out, uint64_t* digests_out, uint64_t* total_digest_out, uint64_t* accepted_out,
                                    float* ms_out);
+/* Fiat-Shamir over several devices, host pointers: same arguments and bytes as pbh_prove_fs_batch / pbh_verify_fs_batch /
+ * pbh_prove_fs_packed / pbh_verify_fs_packed, shard d through device d's entry point on its own host thread. */
+int pbh_multi_prove_fs_batch(pbh_multi* m, size_t n, const uint8_t* wit, size_t wit_pitch, const uint8_t* rand, size_t rand_pitch,
+                             uint8_t* proof, size_t proof_pitch, uint8_t* status, uint8_t* chal_out, size_t chal_pitch);
+int pbh_multi_verify_fs_batch(pbh_multi* m, size_t n, const uint8_t* proof, size_t proof_pitch, uint8_t* result,
+                              uint8_t* chal_out, size_t chal_pitch, uint8_t* gt, size_t gt_pitch);
+int pbh_multi_prove_fs_packed(pbh_multi* m, size_t n, const pbh_packed_fs_witness* in, pbh_packed_proof* out, uint32_t* chal_u_out);
+int pbh_multi_verify_fs_packed(pbh_multi* m, size_t n, const pbh_packed_proof* proofs, uint8_t* result);
+/* pbh_multi_prove_verify_sharded with the Fiat-Shamir transcript: per shard pbh_generate_inputs_dev (its challenge and u planes
+ * are not used), pbh_prove_fs_digest_batch_dev (chal_out = NULL), pbh_verify_fs_bitmap_batch_dev, then the same all-gather.
+ * Outputs as there; bitmap_out and the digests equal what one device computes alone for the same global index range. */
+int pbh_multi_prove_verify_fs_sharded(pbh_multi* m, uint64_t n_total, uint64_t first_index, uint64_t seed, int dist,
+                                      uint8_t* bitmap_out, uint64_t* digests_out, uint64_t* total_digest_out,
+                                      uint64_t* accepted_out, float* ms_out);
 
 /* ---- synthetic inputs (SURVEY.md §8d), device pointers ------------------------------------------ */
 #define PBH_DIST_UNIFORM 0   /* attempt k = 0 only: exercises every status class                    */

@@ -1182,31 +1182,67 @@ int pbh_ctx_get_fs_seed(const pbh_ctx* ctx, uint8_t seed[32]) {
     for (int b = 0; b < 4; b++) seed[4 * i + b] = (uint8_t)(ctx->hs.fs_seed[i] >> (24 - 8 * b));
   return PBH_OK;
 }
-static int launch_prove_fs(pbh_ctx* ctx, cudaStream_t st, const ProveFsArgs& F) {
+// digest (nullable): device uint64, overwritten with the digest of the 27 proof planes (items first_index ..).  The FP32 provers
+// add it in the kernel (launch-local record, no memset); the int32 prover has no such instantiation and runs the digest kernel
+// on a zeroed word after it, as launch_prove does off the TMA path.
+static int launch_prove_fs(pbh_ctx* ctx, cudaStream_t st, const ProveFsArgs& F, uint64_t first_index = 0, uint64_t* digest = nullptr) {
   if (F.base.n == 0) return PBH_OK;
   const int grid = grid_for(ctx, F.base.n, 2);
   const FsSeed seed = fs_seed_of(ctx);
   const bool special = ctx->pbh_circuit && ctx->specialise;
+  if (digest && ctx->prover_fp32) {
+    unsigned int* tc = fresh_tile_counter(ctx, st);
+    if (!tc) return fail(ctx, PBH_ERR_UNSUPPORTED, "too many launches captured into CUDA graphs from this context");
+    const FsDigestArgs D{first_index, (unsigned long long*)digest, tc, peer_window_for(ctx, digest, sizeof(uint64_t))};
+    if (ctx->algo == PBH_ALGO_TABLE && special) prove_fs_kernel<ALGO_TABLE, true, true, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, D);
+    else if (ctx->algo == PBH_ALGO_TABLE) prove_fs_kernel<ALGO_TABLE, true, false, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, D);
+    else prove_fs_kernel<ALGO_ARITH, true, false, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, D);
+    ctx->launches++;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return PBH_OK;
+  }
+  const FsDigestArgs none{};
   if (ctx->algo == PBH_ALGO_TABLE) {
-    if (!ctx->prover_fp32) prove_fs_kernel<ALGO_TABLE, false, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F);
-    else if (special) prove_fs_kernel<ALGO_TABLE, true, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F);
-    else prove_fs_kernel<ALGO_TABLE, true, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F);
+    if (!ctx->prover_fp32) prove_fs_kernel<ALGO_TABLE, false, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, none);
+    else if (special) prove_fs_kernel<ALGO_TABLE, true, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, none);
+    else prove_fs_kernel<ALGO_TABLE, true, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, none);
   } else {
-    if (!ctx->prover_fp32) prove_fs_kernel<ALGO_ARITH, false, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F);
-    else prove_fs_kernel<ALGO_ARITH, true, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F);
+    if (!ctx->prover_fp32) prove_fs_kernel<ALGO_ARITH, false, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, none);
+    else prove_fs_kernel<ALGO_ARITH, true, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, none);
   }
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());
+  if (digest) {
+    CUDA_TRY(ctx, cudaMemsetAsync(digest, 0, sizeof(uint64_t), st));
+    PBH_TRY(launch_digest(ctx, st, F.base.n, first_index, 27, F.base.proof, F.base.proof_pitch, digest));
+    return launch_publish(ctx, st, digest, sizeof(uint64_t), peer_window_for(ctx, digest, sizeof(uint64_t)));
+  }
   return PBH_OK;
 }
+// F.base.bitmap (nullable): the verdict bitmap, packed in the kernel when it is 4-byte aligned, by pack_verdicts_kernel after it
+// otherwise (as launch_verify does); with a peer window it is also stored into every peer's.
 static int launch_verify_fs(pbh_ctx* ctx, cudaStream_t st, const VerifyFsArgs& F) {
   if (F.base.n == 0) return PBH_OK;
   const int grid = grid_for(ctx, F.base.n, 2);
   const FsSeed seed = fs_seed_of(ctx);
-  if (ctx->algo == PBH_ALGO_TABLE) verify_fs_kernel<ALGO_TABLE><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, ctx->verifier_fp32 != 0, seed, ctx->d_tables, F);
-  else verify_fs_kernel<ALGO_ARITH><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, false, seed, ctx->d_tables, F);
+  uint8_t* bitmap = F.base.bitmap;
+  const PeerWindow pw = peer_window_for(ctx, bitmap, (F.base.n + 7) / 8);
+  const bool fused = bitmap && ((uintptr_t)bitmap % 4) == 0;
+  if (fused) {
+    if (ctx->algo == PBH_ALGO_TABLE) verify_fs_kernel<ALGO_TABLE, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, ctx->verifier_fp32 != 0, seed, ctx->d_tables, F, pw);
+    else verify_fs_kernel<ALGO_ARITH, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, false, seed, ctx->d_tables, F, pw);
+  } else {
+    if (ctx->algo == PBH_ALGO_TABLE) verify_fs_kernel<ALGO_TABLE><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, ctx->verifier_fp32 != 0, seed, ctx->d_tables, F, PeerWindow{});
+    else verify_fs_kernel<ALGO_ARITH><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, false, seed, ctx->d_tables, F, PeerWindow{});
+  }
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());
+  if (bitmap && !fused) {
+    pack_verdicts_kernel<<<grid_for(ctx, (F.base.n + 7) / 8, 8), kBlock, 0, st>>>(F.base.n, F.base.result, bitmap);
+    ctx->launches++;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return launch_publish(ctx, st, bitmap, (F.base.n + 7) / 8, pw);
+  }
   return PBH_OK;
 }
 
@@ -1228,6 +1264,27 @@ int pbh_verify_fs_batch_dev(pbh_ctx* ctx, size_t n, const uint8_t* proof, size_t
   if (proof_pitch < n || (chal_out && chal_pitch < n) || (gt && gt_pitch < n)) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "pitch < n");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   VerifyFsArgs F{{proof, proof_pitch, nullptr, 0, nullptr, result, gt, gt_pitch, n, nullptr}, chal_out, chal_pitch};
+  return launch_verify_fs(ctx, ctx->compute, F);
+}
+int pbh_prove_fs_digest_batch_dev(pbh_ctx* ctx, size_t n, const uint8_t* wit, size_t wit_pitch, const uint8_t* rnd, size_t rand_pitch,
+                                  uint8_t* proof, size_t proof_pitch, uint8_t* status, uint8_t* chal_out, size_t chal_pitch,
+                                  uint64_t first_index, uint64_t* digest) {
+  CTX_CHECK(ctx);
+  if (!digest) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  if (n == 0) { CUDA_TRY(ctx, cudaMemsetAsync(digest, 0, sizeof(uint64_t), ctx->compute)); return PBH_OK; }
+  if (!wit || !rnd || !proof || !status) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
+  if (wit_pitch < n || rand_pitch < n || proof_pitch < n || (chal_out && chal_pitch < n)) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "pitch < n");
+  ProveFsArgs F{{wit, wit_pitch, rnd, rand_pitch, nullptr, 0, proof, proof_pitch, status, n}, chal_out, chal_pitch};
+  return launch_prove_fs(ctx, ctx->compute, F, first_index, digest);
+}
+int pbh_verify_fs_bitmap_batch_dev(pbh_ctx* ctx, size_t n, const uint8_t* proof, size_t proof_pitch, uint8_t* result, uint8_t* bitmap) {
+  CTX_CHECK(ctx);
+  if (n == 0) return PBH_OK;
+  if (!proof || !result || !bitmap) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
+  if (proof_pitch < n) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "pitch < n");
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  VerifyFsArgs F{{proof, proof_pitch, nullptr, 0, nullptr, result, nullptr, 0, n, bitmap}, nullptr, 0};
   return launch_verify_fs(ctx, ctx->compute, F);
 }
 int pbh_prove_fs_batch(pbh_ctx* ctx, size_t n, const uint8_t* wit, size_t wit_pitch, const uint8_t* rnd, size_t rand_pitch,

@@ -78,6 +78,51 @@ struct PeerWindow {
   long long delta[7];    // peer address = local address + delta[p]
 };
 
+// Digest of one item's 27 proof bytes as store_proof writes them (pbh_digest_dev's definition), from registers: planes
+// 4k..4k+3 per word.  pp: the nine point words' low 16 bits, ee: the seven evaluations, all zero when the status is not 0.
+__device__ __forceinline__ unsigned long long proof_item_digest(uint64_t index, const uint32_t (&pp)[9], uint32_t inf_lo, uint32_t inf_hi,
+                                                                const uint32_t (&ee)[7]) {
+  DigestState d = digest_item_begin(index, 27);
+  digest_item_word(d, pp[0] | (pp[1] << 16));
+  digest_item_word(d, pp[2] | (pp[3] << 16));
+  digest_item_word(d, pp[4] | (pp[5] << 16));
+  digest_item_word(d, pp[6] | (pp[7] << 16));
+  digest_item_word(d, pp[8] | (inf_lo << 16) | (inf_hi << 24));
+  digest_item_word(d, ee[0] | (ee[1] << 8) | (ee[2] << 16) | (ee[3] << 24));
+  digest_item_word(d, ee[4] | (ee[5] << 8) | (ee[6] << 16));
+  return digest_item_end(d);
+}
+
+// A prover's per-thread digest sums -> ONE atomic per block into the launch-local accumulator next to the tile counters
+// (c[2..3], zero when the launch starts, like them): no memset of the digest word is needed in front of the kernel.  2368
+// same-address atomics (one per warp) at the end of a 2^20-item launch serialise in L2 for microseconds; 296 do not.
+// part: kBlock / 32 words of shared memory.  Ends with the block barrier tile_scheduler_leave relies on.
+__device__ __forceinline__ void digest_block_add(unsigned long long acc, unsigned long long* part, unsigned int* c) {
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_down_sync(0xFFFFFFFFu, acc, o);
+  if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    unsigned long long sum = 0;
+#pragma unroll
+    for (int k = 0; k < kBlock / 32; k++) sum += part[k];
+    atomicAdd(reinterpret_cast<unsigned long long*>(c + 2), sum);
+  }
+}
+// Thread 0 of the last block to leave (tile_scheduler_leave; every block's digest atomic precedes the fence there): every block
+// has added its share, so it publishes the launch's digest (overwriting *digest_out), re-arms the accumulator for the next launch
+// that is handed this record, and pushes the digest to every peer's window.
+__device__ __forceinline__ void digest_publish(unsigned int* c, unsigned long long* digest_out, const PeerWindow& PW) {
+  __threadfence();
+  volatile unsigned long long* acc = reinterpret_cast<volatile unsigned long long*>(c + 2);
+  const unsigned long long d = *acc;
+  *acc = 0ull;
+  *digest_out = d;
+#pragma unroll
+  for (uint32_t p = 0; p < 7; p++)     // fixed trip count: delta[] stays in the parameter bank (no local copy)
+    if (p < PW.n) *reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(digest_out) + PW.delta[p]) = d;
+  __threadfence();
+}
+
 struct ProveArgs {
   const uint8_t* wit; size_t wit_pitch;
   const uint8_t* rnd; size_t rand_pitch;
@@ -171,12 +216,26 @@ struct ProveFsArgs {
   ProveArgs base;                        // chal unused
   uint8_t* chal_out; size_t chal_pitch;  // nullable: 6 planes alpha beta gamma z v u (zero when status != 0)
 };
-template <int ALGO, bool FP32, bool PBH_CIRCUIT>
+// DIGEST instantiation only: the launch's proof digest, by the mechanism of prove_f32_tma_kernel
+struct FsDigestArgs {
+  uint64_t first_index;                  // global index of item 0
+  unsigned long long* digest;            // overwritten by the last block to leave
+  unsigned int* tile_counter;            // the launch-local record (pbh_capi.cu fresh_tile_counter): c[1] and c[2..3] are used
+  PeerWindow PW;
+};
+// DIGEST: a compile-time flag, not a run-time branch, so that the plain instantiations compile as they did (see verify_tma_kernel).
+template <int ALGO, bool FP32, bool PBH_CIRCUIT, bool DIGEST = false>
 __global__ void __launch_bounds__(256, 2) prove_fs_kernel(const Consts K, const ConstsF KF, const FsSeed seed, const Tables* __restrict__ gT,
-                                                           const ProveFsArgs F) {
+                                                           const ProveFsArgs F, const FsDigestArgs D) {
   __shared__ Tables sT;
   stage_tables(sT, gT);
   const ProveArgs& A = F.base;
+  // DIGEST: the thread's running sum lives in shared memory and its slot is found from %tid.x where it is used, so that no
+  // register is held across the item loop for it.  The FP32 provers use all 128 registers two resident blocks allow: with a
+  // register sum the ARITH and generic TABLE instantiations spilled 56 and 32 bytes, with this 44 and 8.
+  __shared__ unsigned long long digest_acc[DIGEST ? 256 : 1];
+  if constexpr (DIGEST) digest_acc[threadIdx.x] = 0;
+  auto slot = [&]() -> unsigned long long& { uint32_t t; asm volatile("mov.u32 %0, %%tid.x;" : "=r"(t)); return digest_acc[t]; };
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < A.n; i += (size_t)gridDim.x * blockDim.x) {
     uint32_t w[12], r[9];
     bool bad = false;
@@ -199,6 +258,25 @@ __global__ void __launch_bounds__(256, 2) prove_fs_kernel(const Consts K, const 
 #pragma unroll
       for (int k = 0; k < 6; k++) F.chal_out[(size_t)k * F.chal_pitch + i] = (uint8_t)(status == 0u ? derived[k] : 0u);
     }
+    if constexpr (DIGEST) {
+      const bool ok = status == 0u;
+      uint32_t pp[9], ee[7], inf_lo = 0, inf_hi = 0;
+#pragma unroll
+      for (int k = 0; k < 9; k++) {
+        const uint32_t pw = ok ? P.pt[k] : 0u;
+        pp[k] = pw & 0xFFFFu;
+        const uint32_t inf = (pw >> 16) & 1u;
+        if (k < 8) inf_lo |= inf << k; else inf_hi |= inf;
+      }
+#pragma unroll
+      for (int k = 0; k < 7; k++) ee[k] = ok ? P.ev[k] : 0u;
+      slot() += proof_item_digest(D.first_index + i, pp, inf_lo, inf_hi, ee);
+    }
+  }
+  if constexpr (DIGEST) {
+    __shared__ unsigned long long part[kBlock / 32];
+    digest_block_add(digest_acc[threadIdx.x], part, D.tile_counter);
+    if (tile_scheduler_leave(D.tile_counter)) digest_publish(D.tile_counter, D.digest, D.PW);
   }
 }
 
@@ -316,21 +394,12 @@ __global__ void __launch_bounds__(kTile, 2) prove_f32_tma_kernel(const __grid_co
     const size_t i = tile * kTile + it;
     if (i < n) status_out[i] = (uint8_t)status;
     if (digest_out != nullptr && i < n) {
-      // digest of this item's 27 proof bytes (pbh_digest_dev's definition), from registers: planes 4k..4k+3 per word
       uint32_t pp[9], ee[7];
 #pragma unroll
       for (int k = 0; k < 9; k++) pp[k] = ok ? (P.pt[k] & 0xFFFFu) : 0u;
 #pragma unroll
       for (int k = 0; k < 7; k++) ee[k] = ok ? P.ev[k] : 0u;
-      DigestState d = digest_item_begin(first_index + i, 27);
-      digest_item_word(d, pp[0] | (pp[1] << 16));
-      digest_item_word(d, pp[2] | (pp[3] << 16));
-      digest_item_word(d, pp[4] | (pp[5] << 16));
-      digest_item_word(d, pp[6] | (pp[7] << 16));
-      digest_item_word(d, pp[8] | (inf_lo << 16) | (inf_hi << 24));
-      digest_item_word(d, ee[0] | (ee[1] << 8) | (ee[2] << 16) | (ee[3] << 24));
-      digest_item_word(d, ee[4] | (ee[5] << 8) | (ee[6] << 16));
-      digest_acc += digest_item_end(d);
+      digest_acc += proof_item_digest(first_index + i, pp, inf_lo, inf_hi, ee);
     }
 
     // TMA clips the item dimension at 16-byte granularity (measured), so a partial last tile whose end is not 16-byte
@@ -351,35 +420,9 @@ __global__ void __launch_bounds__(kTile, 2) prove_f32_tma_kernel(const __grid_co
     }
   }
   if (tid == 0) tma::store_wait_all();
-  if (digest_out != nullptr) {
-    // ONE atomic per block: 2368 same-address atomics (one per warp) at the end of a 2^20-item launch serialise in L2 for
-    // microseconds; 296 do not
-    for (int o = 16; o > 0; o >>= 1) digest_acc += __shfl_down_sync(0xFFFFFFFFu, digest_acc, o);
-    if ((tid & 31) == 0) S.digest_part[tid >> 5] = digest_acc;
-    __syncthreads();
-    if (tid == 0) {
-      unsigned long long sum = 0;
-#pragma unroll
-      for (int k = 0; k < kTile / 32; k++) sum += S.digest_part[k];
-      // into the launch-local accumulator next to the tile counters (zero when the launch starts, like them): no memset of
-      // *digest_out is needed in front of the kernel
-      atomicAdd(reinterpret_cast<unsigned long long*>(tile_counter + 2), sum);
-    }
-  }
+  if (digest_out != nullptr) digest_block_add(digest_acc, S.digest_part, tile_counter);
   const bool last = tile_scheduler_leave(tile_counter);              // thread 0: its digest atomic precedes the fence in leave
-  if (last && digest_out != nullptr) {
-    // every block has added its share: the last one publishes the launch's digest (overwriting *digest_out), re-arms the
-    // accumulator for the next launch that is handed this record, and pushes the digest to every peer's window
-    __threadfence();
-    volatile unsigned long long* acc = reinterpret_cast<volatile unsigned long long*>(tile_counter + 2);
-    const unsigned long long d = *acc;
-    *acc = 0ull;
-    *digest_out = d;
-#pragma unroll
-    for (uint32_t p = 0; p < 7; p++)     // fixed trip count: delta[] stays in the parameter bank (no local copy)
-      if (p < PW.n) *reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(digest_out) + PW.delta[p]) = d;
-    __threadfence();
-  }
+  if (last && digest_out != nullptr) digest_publish(tile_counter, digest_out, PW);
 }
 
 struct VerifyArgs {
@@ -389,7 +432,7 @@ struct VerifyArgs {
   uint8_t* result;
   uint8_t* gt; size_t gt_pitch;   // nullable
   size_t n;
-  uint8_t* bitmap;                // nullable, 4-byte aligned: verdict bit of item i -> bit i%8 of byte i/8 (TMA kernel only)
+  uint8_t* bitmap;                // nullable, 4-byte aligned: verdict bit of item i -> bit i%8 of byte i/8 (TMA kernel, BITMAP verify_fs_kernel)
 };
 
 // Plonk::verify, src/plonk.rs:468-650
@@ -426,13 +469,24 @@ struct VerifyFsArgs {
   VerifyArgs base;                       // chal, u, bitmap unused
   uint8_t* chal_out; size_t chal_pitch;  // nullable: 6 planes alpha beta gamma z v u (zero for PBH_VR_BAD_ENCODING)
 };
-template <int ALGO>
+// 32 verdict bits of the items w0 .. w0 + 31 (ballot word, little endian) into bitmap bytes w0 / 8 ..; only the bytes of items < n
+__device__ __forceinline__ void store_bitmap_word(uint8_t* dst, uint32_t bits, size_t w0, size_t n) {
+  if (w0 + 32 <= n) {
+    *reinterpret_cast<uint32_t*>(dst) = bits;
+  } else {
+    for (size_t b = 0; b < (n - w0 + 7) / 8; b++) dst[b] = (uint8_t)(bits >> (8 * b));
+  }
+}
+// BITMAP: the instantiation that also packs the verdict bits into F.base.bitmap (4-byte aligned) and stores every word at the same
+// offset of each peer's window.  Its grid-stride loop is warp-uniform so that every iteration ballots 32 consecutive items.  A
+// compile-time flag: the plain instantiations compile as they did (see verify_tma_kernel's PEERS).
+template <int ALGO, bool BITMAP = false>
 __global__ void __launch_bounds__(256, 2) verify_fs_kernel(const Consts K, const ConstsF KF, const bool fp32, const FsSeed seed,
-                                                            const Tables* __restrict__ gT, const VerifyFsArgs F) {
+                                                            const Tables* __restrict__ gT, const VerifyFsArgs F, const PeerWindow PW) {
   __shared__ Tables sT;
   stage_tables(sT, gT);
   const VerifyArgs& A = F.base;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < A.n; i += (size_t)gridDim.x * blockDim.x) {
+  auto verify_item = [&](size_t i) -> uint32_t {
     uint32_t px[9], py[9], ev[7];
 #pragma unroll
     for (int k = 0; k < 9; k++) {
@@ -453,6 +507,25 @@ __global__ void __launch_bounds__(256, 2) verify_fs_kernel(const Consts K, const
     if (F.chal_out) {
 #pragma unroll
       for (int k = 0; k < 6; k++) F.chal_out[(size_t)k * F.chal_pitch + i] = (uint8_t)derived[k];
+    }
+    return res;
+  };
+  if constexpr (!BITMAP) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < A.n; i += (size_t)gridDim.x * blockDim.x) verify_item(i);
+  } else {
+    const int lane = threadIdx.x & 31;
+    for (size_t base = (size_t)blockIdx.x * blockDim.x; base < A.n; base += (size_t)gridDim.x * blockDim.x) {
+      const size_t i = base + threadIdx.x;
+      const bool active = i < A.n;
+      const uint32_t res = active ? verify_item(i) : 0u;
+      const uint32_t bits = __ballot_sync(0xFFFFFFFFu, active && (res & 1u));
+      const size_t w0 = i - lane;                   // first item of this warp: a multiple of 32
+      if (lane == 0 && w0 < A.n) {
+        store_bitmap_word(A.bitmap + w0 / 8, bits, w0, A.n);
+#pragma unroll
+        for (uint32_t p = 0; p < 7; p++)            // fixed trip count: delta[] stays in the parameter bank
+          if (p < PW.n) store_bitmap_word(A.bitmap + w0 / 8 + PW.delta[p], bits, w0, A.n);
+      }
     }
   }
 }

@@ -205,8 +205,58 @@ int pbh_multi_verify_packed(pbh_multi* m, size_t n, const pbh_packed_proof* proo
   return for_each_shard(m, n, [&](pbh_ctx* ctx, size_t lo, size_t cnt) { return pbh_verify_packed(ctx, cnt, proofs + lo, chal_u + lo, result + lo); });
 }
 
-int pbh_multi_prove_verify_sharded(pbh_multi* m, uint64_t n_total, uint64_t first_index, uint64_t seed, int dist, uint8_t* bitmap_out,
-                                   uint64_t* digests_out, uint64_t* total_digest_out, uint64_t* accepted_out, float* ms_out) {
+int pbh_multi_prove_fs_batch(pbh_multi* m, size_t n, const uint8_t* wit, size_t wit_pitch, const uint8_t* rnd, size_t rand_pitch,
+                             uint8_t* proof, size_t proof_pitch, uint8_t* status, uint8_t* chal_out, size_t chal_pitch) {
+  if (!m) return PBH_ERR_BAD_ARGUMENT;
+  if (n == 0) return PBH_OK;
+  if (!wit || !rnd || !proof || !status) return mfail(m, PBH_ERR_BAD_ARGUMENT, "null pointer");
+  return for_each_shard(m, n, [&](pbh_ctx* ctx, size_t lo, size_t cnt) {
+    return pbh_prove_fs_batch(ctx, cnt, wit + lo, wit_pitch, rnd + lo, rand_pitch, proof + lo, proof_pitch, status + lo,
+                              chal_out ? chal_out + lo : nullptr, chal_pitch);
+  });
+}
+
+int pbh_multi_verify_fs_batch(pbh_multi* m, size_t n, const uint8_t* proof, size_t proof_pitch, uint8_t* result, uint8_t* chal_out,
+                              size_t chal_pitch, uint8_t* gt, size_t gt_pitch) {
+  if (!m) return PBH_ERR_BAD_ARGUMENT;
+  if (n == 0) return PBH_OK;
+  if (!proof || !result) return mfail(m, PBH_ERR_BAD_ARGUMENT, "null pointer");
+  return for_each_shard(m, n, [&](pbh_ctx* ctx, size_t lo, size_t cnt) {
+    return pbh_verify_fs_batch(ctx, cnt, proof + lo, proof_pitch, result + lo, chal_out ? chal_out + lo : nullptr, chal_pitch,
+                               gt ? gt + lo : nullptr, gt_pitch);
+  });
+}
+
+int pbh_multi_prove_fs_packed(pbh_multi* m, size_t n, const pbh_packed_fs_witness* in, pbh_packed_proof* out, uint32_t* chal_u_out) {
+  if (!m) return PBH_ERR_BAD_ARGUMENT;
+  if (n == 0) return PBH_OK;
+  if (!in || !out) return mfail(m, PBH_ERR_BAD_ARGUMENT, "null pointer");
+  return for_each_shard(m, n, [&](pbh_ctx* ctx, size_t lo, size_t cnt) {
+    return pbh_prove_fs_packed(ctx, cnt, in + lo, out + lo, chal_u_out ? chal_u_out + lo : nullptr);
+  });
+}
+
+int pbh_multi_verify_fs_packed(pbh_multi* m, size_t n, const pbh_packed_proof* proofs, uint8_t* result) {
+  if (!m) return PBH_ERR_BAD_ARGUMENT;
+  if (n == 0) return PBH_OK;
+  if (!proofs || !result) return mfail(m, PBH_ERR_BAD_ARGUMENT, "null pointer");
+  return for_each_shard(m, n, [&](pbh_ctx* ctx, size_t lo, size_t cnt) { return pbh_verify_fs_packed(ctx, cnt, proofs + lo, result + lo); });
+}
+
+}  // extern "C"
+
+// Per-device planes of the sharded pass in Shard::buf (pitch P = Shard::cap items).
+struct ShardPlanes {
+  uint8_t *wit, *rnd, *chal, *u, *proof, *status, *result;
+  size_t P;
+};
+
+// The sharded pass of pbh_multi_prove_verify_sharded and pbh_multi_prove_verify_fs_sharded: sizes the per-device buffers, enqueues
+// `shard(ctx, planes, first, cnt, bitmap, digest)` on every device (it generates, proves with the fused digest and verifies with
+// the fused bitmap), all-gathers the summaries and reads them back from device 0.
+template <class ShardPass>
+static int sharded_pass(pbh_multi* m, uint64_t n_total, uint64_t first_index, uint8_t* bitmap_out, uint64_t* digests_out,
+                        uint64_t* total_digest_out, uint64_t* accepted_out, float* ms_out, ShardPass shard) {
   if (!m) return PBH_ERR_BAD_ARGUMENT;
   if (!bitmap_out) return mfail(m, PBH_ERR_BAD_ARGUMENT, "null pointer");
   const size_t n_dev = m->shards.size();
@@ -229,14 +279,11 @@ int pbh_multi_prove_verify_sharded(pbh_multi* m, uint64_t n_total, uint64_t firs
     MCUDA(m, cudaSetDevice(s.device));
     cudaStream_t st = (cudaStream_t)pbh_ctx_stream(s.ctx);
     const size_t P = s.cap;
-    uint8_t *wit = s.buf, *rnd = s.buf + 12 * P, *chal = s.buf + 21 * P, *u = s.buf + 26 * P, *proof = s.buf + 27 * P, *status = s.buf + 54 * P,
-            *result = s.buf + 55 * P;
+    const ShardPlanes sp{s.buf, s.buf + 12 * P, s.buf + 21 * P, s.buf + 26 * P, s.buf + 27 * P, s.buf + 54 * P, s.buf + 55 * P, P};
     MCUDA(m, cudaEventRecord(s.t0, st));
     MCUDA(m, cudaMemsetAsync(s.summary, 0, per / 8 + 8, st));
     if (cnt) {
-      int rc = pbh_generate_inputs_dev(s.ctx, cnt, first_index + lo, seed, dist, wit, P, rnd, P, chal, P, u, nullptr);
-      if (!rc) rc = pbh_prove_digest_batch_dev(s.ctx, cnt, wit, P, rnd, P, chal, P, proof, P, status, first_index + lo, (uint64_t*)(s.summary + per / 8));
-      if (!rc) rc = pbh_verify_bitmap_batch_dev(s.ctx, cnt, proof, P, chal, P, u, result, s.summary);
+      int rc = shard(s.ctx, sp, first_index + lo, (size_t)cnt, s.summary, (uint64_t*)(s.summary + per / 8));
       if (rc) return mfail(m, rc, std::string("device ") + std::to_string(s.device) + ": " + pbh_last_error(s.ctx));
     }
   }
@@ -282,6 +329,32 @@ int pbh_multi_prove_verify_sharded(pbh_multi* m, uint64_t n_total, uint64_t firs
   if (accepted_out) *accepted_out = accepted;
   if (ms_out) *ms_out = ms;
   return PBH_OK;
+}
+
+
+extern "C" {
+
+int pbh_multi_prove_verify_sharded(pbh_multi* m, uint64_t n_total, uint64_t first_index, uint64_t seed, int dist, uint8_t* bitmap_out,
+                                   uint64_t* digests_out, uint64_t* total_digest_out, uint64_t* accepted_out, float* ms_out) {
+  return sharded_pass(m, n_total, first_index, bitmap_out, digests_out, total_digest_out, accepted_out, ms_out,
+                      [&](pbh_ctx* ctx, const ShardPlanes& p, uint64_t first, size_t cnt, uint8_t* bitmap, uint64_t* digest) {
+                        int rc = pbh_generate_inputs_dev(ctx, cnt, first, seed, dist, p.wit, p.P, p.rnd, p.P, p.chal, p.P, p.u, nullptr);
+                        if (!rc) rc = pbh_prove_digest_batch_dev(ctx, cnt, p.wit, p.P, p.rnd, p.P, p.chal, p.P, p.proof, p.P, p.status, first, digest);
+                        if (!rc) rc = pbh_verify_bitmap_batch_dev(ctx, cnt, p.proof, p.P, p.chal, p.P, p.u, p.result, bitmap);
+                        return rc;
+                      });
+}
+
+int pbh_multi_prove_verify_fs_sharded(pbh_multi* m, uint64_t n_total, uint64_t first_index, uint64_t seed, int dist, uint8_t* bitmap_out,
+                                      uint64_t* digests_out, uint64_t* total_digest_out, uint64_t* accepted_out, float* ms_out) {
+  return sharded_pass(m, n_total, first_index, bitmap_out, digests_out, total_digest_out, accepted_out, ms_out,
+                      [&](pbh_ctx* ctx, const ShardPlanes& p, uint64_t first, size_t cnt, uint8_t* bitmap, uint64_t* digest) {
+                        // the generated challenge and u planes are not used: the transcript derives them
+                        int rc = pbh_generate_inputs_dev(ctx, cnt, first, seed, dist, p.wit, p.P, p.rnd, p.P, p.chal, p.P, p.u, nullptr);
+                        if (!rc) rc = pbh_prove_fs_digest_batch_dev(ctx, cnt, p.wit, p.P, p.rnd, p.P, p.proof, p.P, p.status, nullptr, 0, first, digest);
+                        if (!rc) rc = pbh_verify_fs_bitmap_batch_dev(ctx, cnt, p.proof, p.P, p.result, bitmap);
+                        return rc;
+                      });
 }
 
 }  // extern "C"

@@ -55,7 +55,8 @@ pbh_prove_packed pbh_verify_packed pbh_prove_packed_async pbh_verify_packed_asyn
 pbh_pack_proof_dev pbh_unpack_proof_dev pbh_pack_witness_host pbh_unpack_witness_host pbh_pack_chal_u_host pbh_pack_proofs_host
 pbh_unpack_proofs_host pbh_window_create pbh_window_attach pbh_window_attach_ptrs pbh_window_share pbh_window_destroy pbh_multi_prove_packed pbh_multi_verify_packed pbh_prove_verify_packed_async pbh_host_alloc_input
 pbh_prove_fs_packed pbh_verify_fs_packed pbh_prove_fs_packed_async pbh_verify_fs_packed_async pbh_prove_fs_packed_dev pbh_verify_fs_packed_dev
-pbh_pack_fs_witness_host pbh_unpack_fs_witness_host""".split()
+pbh_pack_fs_witness_host pbh_unpack_fs_witness_host pbh_prove_fs_digest_batch_dev pbh_verify_fs_bitmap_batch_dev pbh_multi_prove_fs_batch
+pbh_multi_verify_fs_batch pbh_multi_prove_fs_packed pbh_multi_verify_fs_packed pbh_multi_prove_verify_fs_sharded""".split()
 
 
 # 32-byte records of include/pbh_b200.h
@@ -588,6 +589,38 @@ class Context:
         if G: out.append(G.arr)
         return out[0] if len(out) == 1 else tuple(out)
 
+    def prove_fs_digest_batch(self, wit, rand, proof, status, digest, first_index=0, chal=None):
+        """Device tensors: prove_fs_batch and the additive digest of the 27 proof planes (== digest(proof, first_index)), fused
+        into the FP32 provers.  `digest`: int64 tensor of one element, overwritten.  chal (6,n): optional derived challenges."""
+        W = _Planes(wit, 12, name="wit"); n = W.n
+        R = _Planes(rand, 9, n, "rand")
+        P = _Planes(proof, 27, n, "proof", out=True); S = _Planes(status, 1, n, "status", out=True)
+        Ch = _Planes(chal, 6, n, "chal", out=True) if chal is not None else None
+        if not (W.dev and R.dev and P.dev and S.dev and (Ch is None or Ch.dev)):
+            raise PbhError("prove_fs_digest_batch takes CUDA tensors")
+        cur = self._dev_begin()
+        rc = self.lib.pbh_prove_fs_digest_batch_dev(self.h, C.c_size_t(n), C.c_void_p(W.ptr), C.c_size_t(W.pitch), C.c_void_p(R.ptr),
+                                                    C.c_size_t(R.pitch), C.c_void_p(P.ptr), C.c_size_t(P.pitch), C.c_void_p(S.ptr),
+                                                    C.c_void_p(Ch.ptr if Ch else None), C.c_size_t(Ch.pitch if Ch else 0),
+                                                    C.c_uint64(first_index), C.c_void_p(digest.data_ptr()))
+        self._dev_end(cur)
+        self._check(rc, "pbh_prove_fs_digest_batch_dev")
+        return P.arr, S.arr.reshape(-1), digest
+
+    def verify_fs_bitmap_batch(self, proof, result, bitmap):
+        """Device tensors: verify_fs_batch and the packed verdict bits (== pack_verdicts(result)), fused when `bitmap` is
+        4-byte aligned."""
+        P = _Planes(proof, 27, name="proof"); n = P.n
+        Rs = _Planes(result, 1, n, "result", out=True)
+        if not (P.dev and Rs.dev):
+            raise PbhError("verify_fs_bitmap_batch takes CUDA tensors")
+        cur = self._dev_begin()
+        rc = self.lib.pbh_verify_fs_bitmap_batch_dev(self.h, C.c_size_t(n), C.c_void_p(P.ptr), C.c_size_t(P.pitch), C.c_void_p(Rs.ptr),
+                                                     C.c_void_p(bitmap.data_ptr()))
+        self._dev_end(cur)
+        self._check(rc, "pbh_verify_fs_bitmap_batch_dev")
+        return Rs.arr.reshape(-1), bitmap
+
     # ---- record (array-of-structs) wire format ----
     def prove_records(self, records):
         """records: numpy array of WITNESS_RECORD (host) -> numpy array of PROOF_RECORD."""
@@ -1085,12 +1118,62 @@ class MultiContext:
 
     def prove_verify_sharded(self, n_total, first_index=0, seed=0xB200, dist=DIST_FULLPATH):
         """-> dict(bitmap uint8[ceil(n/8)], digests uint64[n_dev], total_digest int, accepted int, ms float)."""
+        return self._sharded(self.lib.pbh_multi_prove_verify_sharded, n_total, first_index, seed, dist)
+
+    def prove_verify_fs_sharded(self, n_total, first_index=0, seed=0xB200, dist=DIST_FULLPATH):
+        """prove_verify_sharded with the Fiat-Shamir transcript (the generated challenges are not used); same dict."""
+        return self._sharded(self.lib.pbh_multi_prove_verify_fs_sharded, n_total, first_index, seed, dist)
+
+    def _sharded(self, fn, n_total, first_index, seed, dist):
         bitmap = np.zeros((n_total + 7) // 8, np.uint8); digs = np.zeros(len(self.devices), np.uint64)
         total = C.c_uint64(); acc = C.c_uint64(); ms = C.c_float()
-        rc = self.lib.pbh_multi_prove_verify_sharded(self.h, C.c_uint64(n_total), C.c_uint64(first_index), C.c_uint64(seed), int(dist),
-                                                     C.c_void_p(bitmap.ctypes.data), C.c_void_p(digs.ctypes.data), C.byref(total), C.byref(acc), C.byref(ms))
-        self._check(rc, "pbh_multi_prove_verify_sharded")
+        rc = fn(self.h, C.c_uint64(n_total), C.c_uint64(first_index), C.c_uint64(seed), int(dist), C.c_void_p(bitmap.ctypes.data),
+                C.c_void_p(digs.ctypes.data), C.byref(total), C.byref(acc), C.byref(ms))
+        self._check(rc, fn.__name__)
         return dict(bitmap=bitmap, digests=digs, total_digest=int(total.value), accepted=int(acc.value), ms=float(ms.value))
+
+    # ---- Fiat-Shamir, host arrays: the same bytes as the Context calls ----
+    def prove_fs_batch(self, wit, rand, want_chal=True):
+        """wit (12,n), rand (9,n) -> proof (27,n), status (n,) [, chal (6,n) = alpha beta gamma z v u]."""
+        W = _Planes(wit, 12, name="wit"); n = W.n
+        R = _Planes(rand, 9, n, "rand")
+        proof = np.empty((27, n), np.uint8); status = np.empty((n,), np.uint8); chal = np.empty((6, n), np.uint8) if want_chal else None
+        P = _Planes(proof, 27, n, "proof", out=True); S = _Planes(status, 1, n, "status", out=True)
+        Ch = _Planes(chal, 6, n, "chal", out=True) if want_chal else None
+        rc = self.lib.pbh_multi_prove_fs_batch(self.h, C.c_size_t(n), C.c_void_p(W.ptr), C.c_size_t(W.pitch), C.c_void_p(R.ptr),
+                                               C.c_size_t(R.pitch), C.c_void_p(P.ptr), C.c_size_t(P.pitch), C.c_void_p(S.ptr),
+                                               C.c_void_p(Ch.ptr if Ch else None), C.c_size_t(Ch.pitch if Ch else 0))
+        self._check(rc, "pbh_multi_prove_fs_batch")
+        return (proof, status, chal) if want_chal else (proof, status)
+
+    def verify_fs_batch(self, proof, want_chal=False, want_gt=False):
+        """proof (27,n) -> result (n,) [, chal (6,n)] [, gt (4,n)]."""
+        P = _Planes(proof, 27, name="proof"); n = P.n
+        result = np.empty((n,), np.uint8)
+        chal = np.empty((6, n), np.uint8) if want_chal else None; gt = np.empty((4, n), np.uint8) if want_gt else None
+        Rs = _Planes(result, 1, n, "result", out=True)
+        Ch = _Planes(chal, 6, n, "chal", out=True) if want_chal else None; G = _Planes(gt, 4, n, "gt", out=True) if want_gt else None
+        rc = self.lib.pbh_multi_verify_fs_batch(self.h, C.c_size_t(n), C.c_void_p(P.ptr), C.c_size_t(P.pitch), C.c_void_p(Rs.ptr),
+                                                C.c_void_p(Ch.ptr if Ch else None), C.c_size_t(Ch.pitch if Ch else 0),
+                                                C.c_void_p(G.ptr if G else None), C.c_size_t(G.pitch if G else 0))
+        self._check(rc, "pbh_multi_verify_fs_batch")
+        out = [result] + ([chal] if want_chal else []) + ([gt] if want_gt else [])
+        return out[0] if len(out) == 1 else tuple(out)
+
+    def prove_fs_packed(self, packed_in, want_chal_u=True):
+        """PACKED_FS_WITNESS records -> PACKED_PROOF records [, challenge words]."""
+        pin = Context._packed(packed_in, PACKED_FS_WITNESS, "packed_in"); n = pin.shape[0]
+        out = np.zeros(n, dtype=PACKED_PROOF); cu = np.zeros(n, dtype="<u4") if want_chal_u else None
+        self._check(self.lib.pbh_multi_prove_fs_packed(self.h, C.c_size_t(n), C.c_void_p(pin.ctypes.data), C.c_void_p(out.ctypes.data),
+                                                       C.c_void_p(cu.ctypes.data if want_chal_u else None)), "pbh_multi_prove_fs_packed")
+        return (out, cu) if want_chal_u else out
+
+    def verify_fs_packed(self, proofs):
+        prf = Context._packed(proofs, PACKED_PROOF, "proofs")
+        res = np.zeros(prf.shape[0], dtype=np.uint8)
+        self._check(self.lib.pbh_multi_verify_fs_packed(self.h, C.c_size_t(prf.shape[0]), C.c_void_p(prf.ctypes.data), C.c_void_p(res.ctypes.data)),
+                    "pbh_multi_verify_fs_packed")
+        return res
 
 
 # ================================================================================================

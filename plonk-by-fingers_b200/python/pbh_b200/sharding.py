@@ -6,8 +6,8 @@ only exchange is at the end: an all-gather of each shard's verdict bitmap (1 bit
 bitmaps concatenate (shard boundaries are multiples of 8 items) and digests add modulo 2^64.
 
 `compute(first_index, count)` does the per-shard work and returns (bitmap uint8 tensor of ceil(count/8) bytes,
-digest int64 tensor of 1 element).  On a GPU rank it is `gpu_compute(ctx, ...)` below (CUDA kernels through the C
-ABI); the CPU tests pass an oracle-backed stand-in to exercise this host logic under gloo.
+digest int64 tensor of 1 element).  On a GPU rank it is `gpu_compute(ctx, ...)` below, or `gpu_compute_fs(ctx, ...)` for
+the Fiat-Shamir transcript (CUDA kernels through the C ABI); the CPU tests pass an oracle-backed stand-in to exercise this host logic under gloo.
 """
 import torch
 
@@ -61,6 +61,22 @@ def gpu_compute(ctx, first_index, count, seed=0xB200, dist_kind=1):
     digest = torch.empty((1,), dtype=torch.int64, device=dev)
     ctx.prove_digest_batch(w, r, c, proof, status, digest, first_index=first_index)   # digest fused into the prover
     ctx.verify_bitmap_batch(proof, c, u, result, bitmap)                              # bitmap fused into the verifier
+    ctx.sync()
+    return bitmap, digest
+
+
+def gpu_compute_fs(ctx, first_index, count, seed=0xB200, dist_kind=1):
+    """gpu_compute with the Fiat-Shamir transcript: the challenges and u are derived from the proofs, so the generated ones
+    are not used."""
+    w, r, _, _ = ctx.generate_inputs(count, first_index=first_index, seed=seed, dist=dist_kind)
+    import torch
+    dev = w.device
+    proof = torch.empty((27, count), dtype=torch.uint8, device=dev); status = torch.empty((count,), dtype=torch.uint8, device=dev)
+    result = torch.empty((count,), dtype=torch.uint8, device=dev)
+    bitmap = torch.empty(((count + 7) // 8 + 3) // 4 * 4, dtype=torch.uint8, device=dev)[: (count + 7) // 8]
+    digest = torch.empty((1,), dtype=torch.int64, device=dev)
+    ctx.prove_fs_digest_batch(w, r, proof, status, digest, first_index=first_index)
+    ctx.verify_fs_bitmap_batch(proof, result, bitmap)
     ctx.sync()
     return bitmap, digest
 

@@ -149,6 +149,22 @@ extern "C" {
     pub fn pbh_multi_prove_verify_sharded(m: *mut pbh_multi, n_total: u64, first_index: u64, seed: u64, dist: c_int,
                                           bitmap_out: *mut u8, digests_out: *mut u64, total_digest_out: *mut u64,
                                           accepted_out: *mut u64, ms_out: *mut c_float) -> c_int;
+    // Fiat-Shamir shard summaries (device pointers, compute stream) and the Fiat-Shamir multi-device calls
+    pub fn pbh_prove_fs_digest_batch_dev(ctx: *mut pbh_ctx, n: usize, wit: *const u8, wit_pitch: usize, rand: *const u8, rand_pitch: usize,
+                                         proof: *mut u8, proof_pitch: usize, status: *mut u8, chal_out: *mut u8, chal_pitch: usize,
+                                         first_index: u64, digest: *mut u64) -> c_int;
+    pub fn pbh_verify_fs_bitmap_batch_dev(ctx: *mut pbh_ctx, n: usize, proof: *const u8, proof_pitch: usize, result: *mut u8,
+                                          bitmap: *mut u8) -> c_int;
+    pub fn pbh_multi_prove_fs_batch(m: *mut pbh_multi, n: usize, wit: *const u8, wit_pitch: usize, rand: *const u8, rand_pitch: usize,
+                                    proof: *mut u8, proof_pitch: usize, status: *mut u8, chal_out: *mut u8, chal_pitch: usize) -> c_int;
+    pub fn pbh_multi_verify_fs_batch(m: *mut pbh_multi, n: usize, proof: *const u8, proof_pitch: usize, result: *mut u8,
+                                     chal_out: *mut u8, chal_pitch: usize, gt: *mut u8, gt_pitch: usize) -> c_int;
+    pub fn pbh_multi_prove_fs_packed(m: *mut pbh_multi, n: usize, input: *const PackedFsWitness, out: *mut PackedProof,
+                                     chal_u_out: *mut u32) -> c_int;
+    pub fn pbh_multi_verify_fs_packed(m: *mut pbh_multi, n: usize, proofs: *const PackedProof, result: *mut u8) -> c_int;
+    pub fn pbh_multi_prove_verify_fs_sharded(m: *mut pbh_multi, n_total: u64, first_index: u64, seed: u64, dist: c_int,
+                                             bitmap_out: *mut u8, digests_out: *mut u64, total_digest_out: *mut u64,
+                                             accepted_out: *mut u64, ms_out: *mut c_float) -> c_int;
 }
 
 #[repr(C)]
