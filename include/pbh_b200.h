@@ -207,7 +207,10 @@ int pbh_verify_batch_dev(pbh_ctx* ctx, size_t n, const uint8_t* proof, size_t pr
  * travels beside the upload of the next.  Every buffer must stay valid and untouched until pbh_lane_sync(ctx, lane) or
  * pbh_ctx_sync(ctx) returns.  Only page-locked buffers (pbh_host_alloc, cudaHostAlloc, cudaHostRegister) are asynchronous
  * (PBH_OPT_LANE_MODE says how they travel); with pageable memory the call waits for the context's earlier work and then
- * behaves exactly like the synchronous entry point.  Batches above 2^24 items are processed synchronously as well. */
+ * behaves exactly like the synchronous entry point.  Batches above 2^24 items are processed synchronously as well.
+ * Every lane call (the _async entry points here and below) has one failure policy: a call that fails after it has enqueued
+ * copies of the caller's buffers waits for its lane before it returns the error, so the buffers may be released or reused as
+ * soon as a failed call has returned. */
 #define PBH_LANES 4
 int pbh_prove_batch_async(pbh_ctx* ctx, int lane, size_t n, const uint8_t* wit, size_t wit_pitch, const uint8_t* rand,
                           size_t rand_pitch, const uint8_t* chal, size_t chal_pitch, uint8_t* proof, size_t proof_pitch,

@@ -10,6 +10,8 @@
 #include <unistd.h>
 
 #include <algorithm>
+#include <initializer_list>
+#include <type_traits>
 #include <condition_variable>
 #include <thread>
 #include <vector>
@@ -695,10 +697,72 @@ static int ensure_slots(pbh_ctx* ctx, size_t bytes_per_item) {
 // cycle through kSlots staging buffers, each with its own stream, so the upload of chunk k+2, the kernels of chunk k+1
 // and the download of chunk k overlap.  `body(lo, m, C, base, stream)` enqueues one chunk of m items starting at item
 // lo into the staging buffer `base` (planes of pitch C) on `stream`.
-// Every body lays its planes out inside kStagePlanes rows of C bytes; the static_asserts next to each body tie its
-// plane offsets to this budget.
 static constexpr size_t kStagePlanes = 128;
-static bool host_pinned(const uint8_t* p);
+
+// ---- staging rows ----------------------------------------------------------------------------------------------------------
+// A body lays its buffers out in rows of C bytes of a staging slot (kStagePlanes rows) or of a lane buffer (the kRows its lane
+// call asks for, see lane_call).  Every row range a body uses is named here and nowhere else; the asserts are derived from the names.
+struct Rows {
+  size_t at, count;
+  constexpr size_t end() const { return at + count; }
+};
+template <class... R>
+static constexpr size_t rows_end(R... r) { return std::max({r.end()...}); }
+template <class... R>
+static constexpr bool rows_disjoint(Rows a, R... r) {   // pairwise
+  if constexpr (sizeof...(R) == 0) return true;
+  else return ((a.end() <= r.at || r.end() <= a.at) && ...) && rows_disjoint(r...);
+}
+template <class T = uint8_t>
+static T* at_row(uint8_t* base, size_t C, Rows r) { return reinterpret_cast<T*>(base + r.at * C); }
+
+// byte-plane prover, and the verifier fused behind it (pbh_prove_verify_batch, packed_prove_body); also pbh_prove_records
+struct ProveRows {
+  static constexpr Rows wit{0, 12}, rnd{12, 9}, chal{21, 5}, proof{26, 27}, status{53, 1}, u{54, 1}, res{55, 1};
+  static constexpr size_t kRows = rows_end(wit, rnd, chal, proof, status, u, res);
+};
+// byte-plane verifier (verify_body, packed_verify_body, pbh_verify_records); its proof planes are the prover's rows, where a
+// resident packed verify reads what packed_prove_body left
+struct VerifyRows {
+  static constexpr Rows gt{0, 4}, proof{26, 27}, chal{54, 5}, u{59, 1}, res{60, 1};
+  static constexpr size_t kRows = rows_end(gt, proof, chal, u, res);
+};
+// 32-byte records above the planes (pbh_prove_records, pbh_verify_records)
+struct RecordRows {
+  static constexpr Rows witness{64, 32}, proof{96, 32};
+};
+// packed records above the planes: prover input and output, verifier input (packed proofs, challenge words)
+struct PackedRows {
+  static constexpr Rows in{64, sizeof(pbh_packed_witness)}, out{80, sizeof(pbh_packed_proof)};
+  static constexpr Rows proofs{96, sizeof(pbh_packed_proof)}, chal_u{108, sizeof(uint32_t)};
+  static constexpr size_t kProveRows = std::max(ProveRows::kRows, rows_end(in, out)), kVerifyRows = std::max(VerifyRows::kRows, rows_end(proofs, chal_u));
+};
+// Fiat-Shamir byte planes (pbh_prove_fs_batch, pbh_verify_fs_batch): the prover's or the verifier's rows, and the challenges out
+struct FsRows {
+  static constexpr Rows chal_out{54, 6};
+};
+// Fiat-Shamir packed records: the prover's records, proofs and challenge words; the verifier's proofs and results
+struct FsPackedRows {
+  static constexpr Rows in{64, sizeof(pbh_packed_fs_witness)}, out{80, sizeof(pbh_packed_proof)}, chal_u{92, sizeof(uint32_t)};
+  static constexpr Rows proofs{96, sizeof(pbh_packed_proof)}, res{108, 1};
+  static constexpr size_t kProveRows = rows_end(in, out, chal_u), kVerifyRows = rows_end(proofs, res);
+};
+using PR = ProveRows;
+using VR = VerifyRows;
+static_assert(rows_disjoint(PR::wit, PR::rnd, PR::chal, PR::proof, PR::status, PR::u, PR::res) && rows_disjoint(VR::gt, VR::proof, VR::chal, VR::u, VR::res) &&
+                  rows_disjoint(PR::wit, PR::rnd, PR::proof, PR::status, FsRows::chal_out) && rows_disjoint(VR::gt, VR::proof, VR::res, FsRows::chal_out) &&
+                  rows_disjoint(RecordRows::witness, RecordRows::proof) &&
+                  std::max({PR::kRows, VR::kRows, FsRows::chal_out.end()}) <= std::min(RecordRows::witness.at, PackedRows::in.at),
+              "no body uses a row twice; records sit above the planes");
+static_assert(std::max({PackedRows::kProveRows, PackedRows::kVerifyRows, RecordRows::proof.end(), FsPackedRows::kProveRows, FsPackedRows::kVerifyRows,
+}) <= kStagePlanes,
+              "every body fits a staging slot");
+static_assert(rows_disjoint(PackedRows::in, PackedRows::out, PackedRows::proofs, PackedRows::chal_u) &&
+                  rows_disjoint(FsPackedRows::in, FsPackedRows::out, FsPackedRows::chal_u, FsPackedRows::proofs, FsPackedRows::res),
+              "the prover's and the verifier's packed records are disjoint");
+static_assert(VR::proof.at == PR::proof.at && VR::proof.count == PR::proof.count && rows_disjoint(PR::proof, VR::chal, VR::u, VR::res, PackedRows::chal_u),
+              "resident proofs: packed_verify_body reads the proof planes packed_prove_body left and writes none of them");
+static bool host_pinned(const void* p);
 static int slot_of(const pbh_ctx* ctx, const uint8_t* base) {
   for (int s = 0; s < kSlots; s++)
     if (ctx->slot_buf[s] && ctx->slot_buf[s] == base) return s;
@@ -841,6 +905,60 @@ static uint8_t* mapped_host_alias(pbh_ctx* ctx, const uint8_t* p, size_t span) {
   return (uint8_t*)lo.devicePointer;
 }
 
+// One byte-plane prove of A.n items on st.  Each direction either goes through rows of `base` by the copy engines (A holds the
+// caller's host buffers for it) or is read / written by the kernel in place (A holds device or mapped memory for it).
+static int prove_body(pbh_ctx* ctx, cudaStream_t st, uint8_t* base, size_t C, ProveArgs A, bool stage_in, bool stage_out) {
+  const ProveArgs H = A;
+  if (stage_in) {
+    uint8_t *wit = at_row(base, C, PR::wit), *rnd = at_row(base, C, PR::rnd), *chal = at_row(base, C, PR::chal);
+    PBH_TRY(stage_h2d(ctx, base, st, wit, C, H.wit, H.wit_pitch, A.n, PR::wit.count));
+    PBH_TRY(stage_h2d(ctx, base, st, rnd, C, H.rnd, H.rand_pitch, A.n, PR::rnd.count));
+    PBH_TRY(stage_h2d(ctx, base, st, chal, C, H.chal, H.chal_pitch, A.n, PR::chal.count));
+    A.wit = wit; A.rnd = rnd; A.chal = chal;
+    A.wit_pitch = A.rand_pitch = A.chal_pitch = C;
+  }
+  if (stage_out) { A.proof = at_row(base, C, PR::proof); A.proof_pitch = C; A.status = at_row(base, C, PR::status); }
+  PBH_TRY(launch_prove(ctx, st, A));
+  if (stage_out) {
+    PBH_TRY(stage_d2h(ctx, base, st, H.proof, H.proof_pitch, A.proof, C, A.n, PR::proof.count));
+    PBH_TRY(stage_d2h(ctx, base, st, H.status, 0, A.status, 0, A.n, 1));
+  }
+  return PBH_OK;
+}
+// One byte-plane verify, with the same choice per direction.
+static int verify_body(pbh_ctx* ctx, cudaStream_t st, uint8_t* base, size_t C, VerifyArgs A, bool stage_in, bool stage_out) {
+  const VerifyArgs H = A;
+  if (stage_in) {
+    uint8_t *proof = at_row(base, C, VR::proof), *chal = at_row(base, C, VR::chal), *u = at_row(base, C, VR::u);
+    PBH_TRY(stage_h2d(ctx, base, st, proof, C, H.proof, H.proof_pitch, A.n, VR::proof.count));
+    PBH_TRY(stage_h2d(ctx, base, st, chal, C, H.chal, H.chal_pitch, A.n, VR::chal.count));
+    PBH_TRY(stage_h2d(ctx, base, st, u, 0, H.u, 0, A.n, 1));
+    A.proof = proof; A.chal = chal; A.u = u;
+    A.proof_pitch = A.chal_pitch = C;
+  }
+  if (stage_out) {
+    A.result = at_row(base, C, VR::res);
+    if (A.gt) { A.gt = at_row(base, C, VR::gt); A.gt_pitch = C; }
+  }
+  PBH_TRY(launch_verify(ctx, st, A));
+  if (stage_out) {
+    PBH_TRY(stage_d2h(ctx, base, st, H.result, 0, A.result, 0, A.n, 1));
+    if (H.gt) PBH_TRY(stage_d2h(ctx, base, st, H.gt, H.gt_pitch, A.gt, C, A.n, VR::gt.count));
+  }
+  return PBH_OK;
+}
+// The buffers of A replaced by their mapped device aliases (nullptr where there is none; a null gt stays null)
+static ProveArgs mapped(pbh_ctx* ctx, const ProveArgs& A) {
+  return ProveArgs{mapped_host_alias(ctx, A.wit, 11 * A.wit_pitch + A.n), A.wit_pitch, mapped_host_alias(ctx, A.rnd, 8 * A.rand_pitch + A.n),
+                   A.rand_pitch, mapped_host_alias(ctx, A.chal, 4 * A.chal_pitch + A.n), A.chal_pitch,
+                   mapped_host_alias(ctx, A.proof, 26 * A.proof_pitch + A.n), A.proof_pitch, mapped_host_alias(ctx, A.status, A.n), A.n};
+}
+static VerifyArgs mapped(pbh_ctx* ctx, const VerifyArgs& A) {
+  return VerifyArgs{mapped_host_alias(ctx, A.proof, 26 * A.proof_pitch + A.n), A.proof_pitch, mapped_host_alias(ctx, A.chal, 4 * A.chal_pitch + A.n),
+                    A.chal_pitch, mapped_host_alias(ctx, A.u, A.n), mapped_host_alias(ctx, A.result, A.n),
+                    A.gt ? mapped_host_alias(ctx, A.gt, 3 * A.gt_pitch + A.n) : nullptr, A.gt_pitch, A.n, nullptr};
+}
+
 int pbh_prove_batch(pbh_ctx* ctx, size_t n, const uint8_t* wit, size_t wit_pitch, const uint8_t* rnd, size_t rand_pitch,
                     const uint8_t* chal, size_t chal_pitch, uint8_t* proof, size_t proof_pitch, uint8_t* status) {
   CTX_CHECK(ctx);
@@ -848,30 +966,15 @@ int pbh_prove_batch(pbh_ctx* ctx, size_t n, const uint8_t* wit, size_t wit_pitch
   if (!wit || !rnd || !chal || !proof || !status) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
   if (wit_pitch < n || rand_pitch < n || chal_pitch < n || proof_pitch < n) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "pitch < n");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  int rc;
-  {
-    const uint8_t *a_wit = mapped_host_alias(ctx, wit, 11 * wit_pitch + n), *a_rnd = mapped_host_alias(ctx, rnd, 8 * rand_pitch + n),
-                  *a_chal = mapped_host_alias(ctx, chal, 4 * chal_pitch + n);
-    uint8_t *a_proof = mapped_host_alias(ctx, proof, 26 * proof_pitch + n), *a_status = mapped_host_alias(ctx, status, n);
-    if (a_wit && a_rnd && a_chal && a_proof && a_status) {
-      ProveArgs A{a_wit, wit_pitch, a_rnd, rand_pitch, a_chal, chal_pitch, a_proof, proof_pitch, a_status, n};
-      rc = launch_prove(ctx, ctx->slot_stream[0], A);
-      if (rc) return rc;
-      CUDA_TRY(ctx, cudaStreamSynchronize(ctx->slot_stream[0]));
-      return PBH_OK;
-    }
+  const ProveArgs M = mapped(ctx, ProveArgs{wit, wit_pitch, rnd, rand_pitch, chal, chal_pitch, proof, proof_pitch, status, n});
+  if (M.wit && M.rnd && M.chal && M.proof && M.status) {   // everything mapped: the body in place, one launch
+    PBH_TRY(launch_prove(ctx, ctx->slot_stream[0], M));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->slot_stream[0]));
+    return PBH_OK;
   }
   return for_each_chunk(ctx, n, [&](size_t lo, size_t m, size_t C, uint8_t* base, cudaStream_t st) -> int {
-    uint8_t *d_wit = base, *d_rnd = base + 12 * C, *d_chal = base + 21 * C, *d_proof = base + 26 * C, *d_status = base + 53 * C;
-    PBH_TRY(stage_h2d(ctx, base, st, d_wit, C, wit + lo, wit_pitch, m, 12));
-    PBH_TRY(stage_h2d(ctx, base, st, d_rnd, C, rnd + lo, rand_pitch, m, 9));
-    PBH_TRY(stage_h2d(ctx, base, st, d_chal, C, chal + lo, chal_pitch, m, 5));
-    ProveArgs A{d_wit, C, d_rnd, C, d_chal, C, d_proof, C, d_status, m};
-    int rc = launch_prove(ctx, st, A);
-    if (rc) return rc;
-    PBH_TRY(stage_d2h(ctx, base, st, proof + lo, proof_pitch, d_proof, C, m, 27));
-    PBH_TRY(stage_d2h(ctx, base, st, status + lo, 0, d_status, 0, m, 1));
-    return PBH_OK;
+    const ProveArgs A{wit + lo, wit_pitch, rnd + lo, rand_pitch, chal + lo, chal_pitch, proof + lo, proof_pitch, status + lo, m};
+    return prove_body(ctx, st, base, C, A, true, true);
   });
 }
 
@@ -882,30 +985,15 @@ int pbh_verify_batch(pbh_ctx* ctx, size_t n, const uint8_t* proof, size_t proof_
   if (!proof || !chal || !u || !result) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
   if (proof_pitch < n || chal_pitch < n || (gt && gt_pitch < n)) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "pitch < n");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  int rc;
-  {
-    const uint8_t *a_proof = mapped_host_alias(ctx, proof, 26 * proof_pitch + n), *a_chal = mapped_host_alias(ctx, chal, 4 * chal_pitch + n),
-                  *a_u = mapped_host_alias(ctx, u, n);
-    uint8_t *a_res = mapped_host_alias(ctx, result, n), *a_gt = gt ? mapped_host_alias(ctx, gt, 3 * gt_pitch + n) : nullptr;
-    if (a_proof && a_chal && a_u && a_res && (!gt || a_gt)) {
-      VerifyArgs A{a_proof, proof_pitch, a_chal, chal_pitch, a_u, a_res, a_gt, gt_pitch, n, nullptr};
-      rc = launch_verify(ctx, ctx->slot_stream[0], A);
-      if (rc) return rc;
-      CUDA_TRY(ctx, cudaStreamSynchronize(ctx->slot_stream[0]));
-      return PBH_OK;
-    }
+  const VerifyArgs M = mapped(ctx, VerifyArgs{proof, proof_pitch, chal, chal_pitch, u, result, gt, gt_pitch, n, nullptr});
+  if (M.proof && M.chal && M.u && M.result && (!gt || M.gt)) {
+    PBH_TRY(launch_verify(ctx, ctx->slot_stream[0], M));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->slot_stream[0]));
+    return PBH_OK;
   }
   return for_each_chunk(ctx, n, [&](size_t lo, size_t m, size_t C, uint8_t* base, cudaStream_t st) -> int {
-    uint8_t *d_proof = base, *d_chal = base + 27 * C, *d_u = base + 32 * C, *d_res = base + 33 * C, *d_gt = base + 34 * C;
-    PBH_TRY(stage_h2d(ctx, base, st, d_proof, C, proof + lo, proof_pitch, m, 27));
-    PBH_TRY(stage_h2d(ctx, base, st, d_chal, C, chal + lo, chal_pitch, m, 5));
-    PBH_TRY(stage_h2d(ctx, base, st, d_u, 0, u + lo, 0, m, 1));
-    VerifyArgs A{d_proof, C, d_chal, C, d_u, d_res, gt ? d_gt : nullptr, C, m, nullptr};
-    int rc = launch_verify(ctx, st, A);
-    if (rc) return rc;
-    PBH_TRY(stage_d2h(ctx, base, st, result + lo, 0, d_res, 0, m, 1));
-    if (gt) PBH_TRY(stage_d2h(ctx, base, st, gt + lo, gt_pitch, d_gt, C, m, 4));
-    return PBH_OK;
+    const VerifyArgs A{proof + lo, proof_pitch, chal + lo, chal_pitch, u + lo, result + lo, gt ? gt + lo : nullptr, gt_pitch, m, nullptr};
+    return verify_body(ctx, st, base, C, A, true, true);
   });
 }
 
@@ -920,11 +1008,12 @@ int pbh_prove_verify_batch(pbh_ctx* ctx, size_t n, const uint8_t* wit, size_t wi
   if (wit_pitch < n || rand_pitch < n || chal_pitch < n || proof_pitch < n) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "pitch < n");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   return for_each_chunk(ctx, n, [&](size_t lo, size_t m, size_t C, uint8_t* base, cudaStream_t st) -> int {
-    uint8_t *d_wit = base, *d_rnd = base + 12 * C, *d_chal = base + 21 * C, *d_proof = base + 26 * C, *d_status = base + 53 * C,
-            *d_u = base + 54 * C, *d_res = base + 55 * C;
-    PBH_TRY(stage_h2d(ctx, base, st, d_wit, C, wit + lo, wit_pitch, m, 12));
-    PBH_TRY(stage_h2d(ctx, base, st, d_rnd, C, rnd + lo, rand_pitch, m, 9));
-    PBH_TRY(stage_h2d(ctx, base, st, d_chal, C, chal + lo, chal_pitch, m, 5));
+    uint8_t *d_wit = at_row(base, C, PR::wit), *d_rnd = at_row(base, C, PR::rnd), *d_chal = at_row(base, C, PR::chal),
+            *d_proof = at_row(base, C, PR::proof), *d_status = at_row(base, C, PR::status), *d_u = at_row(base, C, PR::u),
+            *d_res = at_row(base, C, PR::res);
+    PBH_TRY(stage_h2d(ctx, base, st, d_wit, C, wit + lo, wit_pitch, m, PR::wit.count));
+    PBH_TRY(stage_h2d(ctx, base, st, d_rnd, C, rnd + lo, rand_pitch, m, PR::rnd.count));
+    PBH_TRY(stage_h2d(ctx, base, st, d_chal, C, chal + lo, chal_pitch, m, PR::chal.count));
     PBH_TRY(stage_h2d(ctx, base, st, d_u, 0, u + lo, 0, m, 1));
     ProveArgs A{d_wit, C, d_rnd, C, d_chal, C, d_proof, C, d_status, m};
     int rc = launch_prove(ctx, st, A);
@@ -932,42 +1021,27 @@ int pbh_prove_verify_batch(pbh_ctx* ctx, size_t n, const uint8_t* wit, size_t wi
     VerifyArgs V{d_proof, C, d_chal, C, d_u, d_res, nullptr, 0, m, nullptr};
     rc = launch_verify(ctx, st, V);
     if (rc) return rc;
-    PBH_TRY(stage_d2h(ctx, base, st, proof + lo, proof_pitch, d_proof, C, m, 27));
+    PBH_TRY(stage_d2h(ctx, base, st, proof + lo, proof_pitch, d_proof, C, m, PR::proof.count));
     PBH_TRY(stage_d2h(ctx, base, st, status + lo, 0, d_status, 0, m, 1));
     PBH_TRY(stage_d2h(ctx, base, st, result + lo, 0, d_res, 0, m, 1));
     return PBH_OK;
   });
 }
 
-// plane budgets of the staged bodies (rows of C bytes inside one staging slot, see for_each_chunk)
-static_assert(53 + 1 <= kStagePlanes, "pbh_prove_batch: 12 + 9 + 5 + 27 + 1 planes");
-static_assert(34 + 4 <= kStagePlanes, "pbh_verify_batch: 27 + 5 + 1 + 1 + 4 planes");
-static_assert(55 + 1 <= kStagePlanes, "pbh_prove_verify_batch: 54 + u + result");
-static_assert(49 + 6 <= kStagePlanes && 34 + 4 <= kStagePlanes, "Fiat-Shamir bodies");
-static_assert(96 + sizeof(pbh_proof_record) <= kStagePlanes && 64 + sizeof(pbh_witness_record) <= 96, "record bodies: planes below row 64, records above");
-static_assert(64 + sizeof(pbh_packed_witness) <= 80 && 80 + sizeof(pbh_packed_proof) <= 96 && 96 + sizeof(pbh_packed_proof) + 4 <= kStagePlanes,
-              "packed bodies: planes below row 64, packed input 64..79, packed output 80..91, verifier input 96..111");
-
 // ---- asynchronous host-pointer calls (include/pbh_b200.h "lanes") ------------------------------------------------------
-// A lane is one of the context's slot streams.  Page-locked, mapped buffers run in place on the lane's stream and the call
-// returns at once; the grids are half the synchronous ones (one prover block and two verifier blocks per SM), so that
-// kernels of different lanes are resident together and the upload of one batch shares the link with the download of
-// another.  Other buffers take the synchronous staged path (copies from pageable memory are synchronous anyway).
+// A lane is one of the context's slot streams, with a whole-batch staging buffer.  Page-locked buffers travel on the lane's
+// stream and the call returns at once.  Kernels that read or write mapped host memory in place run on half grids (one prover
+// block and two verifier blocks per SM), so that kernels of different lanes are resident together and the upload of one batch
+// shares the link with the download of another.  Other buffers take the synchronous staged path (copies from pageable memory
+// are synchronous anyway).  Calls on one lane run in issue order, so a call may reuse the rows of the lane buffer the previous
+// one used; the proof planes a packed prove leaves there are the one thing a later call (a resident verify) reads.
 static int lane_stream(pbh_ctx* ctx, int lane, cudaStream_t* st) {
   if (lane < 0 || lane >= PBH_LANES) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "lane out of range");
   *st = ctx->slot_stream[lane];
   return PBH_OK;
 }
-// Whatever a lane call does next, the proof planes an earlier prove call left in the lane buffer stop being "the proofs the
-// caller's buffer will hold": every lane entry point and every synchronisation forgets them first.
-static const void* take_resident(pbh_ctx* ctx, int lane, size_t* n) {
-  const void* h = ctx->resident_host[lane];
-  *n = ctx->resident_n[lane];
-  ctx->resident_host[lane] = nullptr;
-  return h;
-}
 // page-locked (mapped or not): the copy engines can read and write it asynchronously
-static bool host_pinned(const uint8_t* p) {
+static bool host_pinned(const void* p) {
   if (!p) return false;
   cudaPointerAttributes a{};
   if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
@@ -984,114 +1058,109 @@ static int ensure_lane(pbh_ctx* ctx, int lane, size_t bytes) {
 }
 static constexpr size_t kLaneMaxItems = (size_t)1 << 24;   // larger batches take the synchronous chunked path
 
+// How a lane call's buffers travel
+struct LanePlan {
+  bool async;      // on the lane; else the call waits for the context and runs synchronously
+  size_t rows;     // lane-buffer rows the body stages through (0: none)
+  bool in_place;   // a kernel reads or writes mapped host memory (half grids)
+};
+// every buffer (null ones aside) page-locked and the batch within kLaneMaxItems: all of it through the lane buffer
+static LanePlan staged_plan(size_t n, size_t rows, std::initializer_list<const void*> bufs) {
+  bool ok = n <= kLaneMaxItems;
+  for (const void* p : bufs) ok = ok && (!p || host_pinned(p));
+  return {ok, rows, false};
+}
+// a byte-plane call (PBH_OPT_LANE_MODE): each direction through the lane buffer by the copy engine (its mode bit set, or
+// page-locked memory that is not mapped) or in place on mapped memory
+static LanePlan plane_plan(const pbh_ctx* ctx, size_t n, size_t rows, bool in_pinned, bool in_mapped, bool out_pinned, bool out_mapped,
+                           bool* stage_in, bool* stage_out) {
+  *stage_in = in_pinned && ((ctx->lane_mode & 1) || !in_mapped) && n <= kLaneMaxItems;
+  *stage_out = out_pinned && ((ctx->lane_mode & 2) || !out_mapped) && n <= kLaneMaxItems;
+  return {(*stage_in || in_mapped) && (*stage_out || out_mapped), (*stage_in || *stage_out) ? rows : 0, !(*stage_in && *stage_out)};
+}
+
+// Every lane call (include/pbh_b200.h "lanes"): the lane is checked and its resident proofs are forgotten; n == 0 returns; `bad`
+// is what is wrong with the caller's arguments, or nullptr.  `plan()` then decides: buffers that cannot travel on the lane take
+// the synchronous call `sync()` once everything enqueued on the context is done (it shares the slot streams with the lanes).
+// Otherwise the lane buffer is grown to plan.rows rows of C = n rounded up to a tile and `body(stream, lane buffer, C, resident)`
+// enqueues the batch; `resident` is the host buffer whose proofs the previous call on the lane left in the lane buffer, when
+// it had this n and the buffer was not reallocated since.  A body that fails may already have enqueued copies of the caller's
+// buffers: the call waits for the lane before it returns the error, since the caller may release them once it has returned.
+template <class Plan, class Body, class Sync>
+static int lane_call(pbh_ctx* ctx, int lane, size_t n, const char* bad, Plan plan, Body body, Sync sync) {
+  cudaStream_t st;
+  PBH_TRY(lane_stream(ctx, lane, &st));
+  const void* resident = ctx->resident_n[lane] == n ? ctx->resident_host[lane] : nullptr;
+  ctx->resident_host[lane] = nullptr;
+  if (n == 0) return PBH_OK;
+  if (bad) return fail(ctx, PBH_ERR_BAD_ARGUMENT, bad);
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  const LanePlan p = plan();
+  if (!p.async) {
+    PBH_TRY(pbh_ctx_sync(ctx));
+    return sync();
+  }
+  const size_t C = (n + kTile - 1) / kTile * kTile;
+  if (p.rows) {
+    const size_t had = ctx->lane_bytes[lane];
+    PBH_TRY(ensure_lane(ctx, lane, p.rows * C));
+    if (ctx->lane_bytes[lane] != had) resident = nullptr;
+  }
+  const int keep = ctx->grid_scale;
+  if (p.in_place) ctx->grid_scale = 1;
+  const int rc = body(st, ctx->lane_buf[lane], C, resident);
+  ctx->grid_scale = keep;
+  if (rc != PBH_OK) {
+    const std::string err = ctx->last_error;
+    cudaStreamSynchronize(st);
+    cudaGetLastError();
+    ctx->last_error = err;
+  }
+  return rc;
+}
+
 int pbh_prove_batch_async(pbh_ctx* ctx, int lane, size_t n, const uint8_t* wit, size_t wit_pitch, const uint8_t* rnd, size_t rand_pitch,
                           const uint8_t* chal, size_t chal_pitch, uint8_t* proof, size_t proof_pitch, uint8_t* status) {
   CTX_CHECK(ctx);
-  cudaStream_t st;
-  int rc = lane_stream(ctx, lane, &st);
-  if (rc) return rc;
-  ctx->resident_host[lane] = nullptr;
-  if (n == 0) return PBH_OK;
-  if (!wit || !rnd || !chal || !proof || !status) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
-  if (wit_pitch < n || rand_pitch < n || chal_pitch < n || proof_pitch < n) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "pitch < n");
-  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  const uint8_t *a_wit = mapped_host_alias(ctx, wit, 11 * wit_pitch + n), *a_rnd = mapped_host_alias(ctx, rnd, 8 * rand_pitch + n),
-                *a_chal = mapped_host_alias(ctx, chal, 4 * chal_pitch + n);
-  uint8_t *a_proof = mapped_host_alias(ctx, proof, 26 * proof_pitch + n), *a_status = mapped_host_alias(ctx, status, n);
-  const bool in_mapped = a_wit && a_rnd && a_chal, out_mapped = a_proof && a_status;
-  const bool in_pinned = host_pinned(wit) && host_pinned(rnd) && host_pinned(chal), out_pinned = host_pinned(proof) && host_pinned(status);
-  // inputs: uploaded by the copy engine (mode bit 0, page-locked memory) or read in place (mapped memory); outputs alike (bit 1)
-  const bool in_ce = in_pinned && ((ctx->lane_mode & 1) || !in_mapped) && n <= kLaneMaxItems;
-  const bool out_ce = out_pinned && ((ctx->lane_mode & 2) || !out_mapped) && n <= kLaneMaxItems;
-  if ((in_ce || in_mapped) && (out_ce || out_mapped)) {
-    const size_t C = (n + kTile - 1) / kTile * kTile;
-    uint8_t* base = nullptr;
-    if (in_ce || out_ce) {
-      rc = ensure_lane(ctx, lane, 64 * C);
-      if (rc) return rc;
-      base = ctx->lane_buf[lane];
-    }
-    ProveArgs A{a_wit, wit_pitch, a_rnd, rand_pitch, a_chal, chal_pitch, a_proof, proof_pitch, a_status, n};
-    if (in_ce) {
-      uint8_t *d_wit = base, *d_rnd = base + 12 * C, *d_chal = base + 21 * C;
-      CUDA_TRY(ctx, cudaMemcpy2DAsync(d_wit, C, wit, wit_pitch, n, 12, cudaMemcpyHostToDevice, st));
-      CUDA_TRY(ctx, cudaMemcpy2DAsync(d_rnd, C, rnd, rand_pitch, n, 9, cudaMemcpyHostToDevice, st));
-      CUDA_TRY(ctx, cudaMemcpy2DAsync(d_chal, C, chal, chal_pitch, n, 5, cudaMemcpyHostToDevice, st));
-      A.wit = d_wit; A.wit_pitch = C; A.rnd = d_rnd; A.rand_pitch = C; A.chal = d_chal; A.chal_pitch = C;
-    }
-    if (out_ce) { A.proof = base + 26 * C; A.proof_pitch = C; A.status = base + 53 * C; }
-    // kernels that touch host memory directly run on half grids, so that two lanes' kernels are resident together
-    const int keep = ctx->grid_scale;
-    ctx->grid_scale = (in_ce && out_ce) ? 2 : 1;
-    rc = launch_prove(ctx, st, A);
-    ctx->grid_scale = keep;
-    if (rc) return rc;
-    if (out_ce) {
-      CUDA_TRY(ctx, cudaMemcpy2DAsync(proof, proof_pitch, A.proof, C, n, 27, cudaMemcpyDeviceToHost, st));
-      CUDA_TRY(ctx, cudaMemcpyAsync(status, A.status, n, cudaMemcpyDeviceToHost, st));
-    }
-    return PBH_OK;
-  }
-  rc = pbh_ctx_sync(ctx);   // the staged path shares the slot streams with the lanes
-  if (rc) return rc;
-  return pbh_prove_batch(ctx, n, wit, wit_pitch, rnd, rand_pitch, chal, chal_pitch, proof, proof_pitch, status);
+  const char* bad = !wit || !rnd || !chal || !proof || !status ? "null pointer"
+                    : wit_pitch < n || rand_pitch < n || chal_pitch < n || proof_pitch < n ? "pitch < n" : nullptr;
+  ProveArgs A{wit, wit_pitch, rnd, rand_pitch, chal, chal_pitch, proof, proof_pitch, status, n};
+  bool stage_in = false, stage_out = false;
+  return lane_call(ctx, lane, n, bad,
+      [&] {
+        const ProveArgs M = mapped(ctx, A);
+        const LanePlan p = plane_plan(ctx, n, PR::kRows, host_pinned(wit) && host_pinned(rnd) && host_pinned(chal), M.wit && M.rnd && M.chal,
+                                      host_pinned(proof) && host_pinned(status), M.proof && M.status, &stage_in, &stage_out);
+        if (!stage_in) { A.wit = M.wit; A.rnd = M.rnd; A.chal = M.chal; }
+        if (!stage_out) { A.proof = M.proof; A.status = M.status; }
+        return p;
+      },
+      [&](cudaStream_t st, uint8_t* base, size_t C, const void*) { return prove_body(ctx, st, base, C, A, stage_in, stage_out); },
+      [&] { return pbh_prove_batch(ctx, n, wit, wit_pitch, rnd, rand_pitch, chal, chal_pitch, proof, proof_pitch, status); });
 }
 int pbh_verify_batch_async(pbh_ctx* ctx, int lane, size_t n, const uint8_t* proof, size_t proof_pitch, const uint8_t* chal,
                            size_t chal_pitch, const uint8_t* u, uint8_t* result, uint8_t* gt, size_t gt_pitch) {
   CTX_CHECK(ctx);
-  cudaStream_t st;
-  int rc = lane_stream(ctx, lane, &st);
-  if (rc) return rc;
-  ctx->resident_host[lane] = nullptr;
-  if (n == 0) return PBH_OK;
-  if (!proof || !chal || !u || !result) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
-  if (proof_pitch < n || chal_pitch < n || (gt && gt_pitch < n)) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "pitch < n");
-  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  const uint8_t *a_proof = mapped_host_alias(ctx, proof, 26 * proof_pitch + n), *a_chal = mapped_host_alias(ctx, chal, 4 * chal_pitch + n),
-                *a_u = mapped_host_alias(ctx, u, n);
-  uint8_t *a_res = mapped_host_alias(ctx, result, n), *a_gt = gt ? mapped_host_alias(ctx, gt, 3 * gt_pitch + n) : nullptr;
-  const bool in_mapped = a_proof && a_chal && a_u, out_mapped = a_res && (!gt || a_gt);
-  const bool in_pinned = host_pinned(proof) && host_pinned(chal) && host_pinned(u), out_pinned = host_pinned(result) && (!gt || host_pinned(gt));
-  const bool in_ce = in_pinned && ((ctx->lane_mode & 1) || !in_mapped) && n <= kLaneMaxItems;
-  const bool out_ce = out_pinned && ((ctx->lane_mode & 2) || !out_mapped) && n <= kLaneMaxItems;
-  if ((in_ce || in_mapped) && (out_ce || out_mapped)) {
-    const size_t C = (n + kTile - 1) / kTile * kTile;
-    uint8_t* base = nullptr;
-    if (in_ce || out_ce) {
-      rc = ensure_lane(ctx, lane, 64 * C);
-      if (rc) return rc;
-      base = ctx->lane_buf[lane];
-    }
-    VerifyArgs A{a_proof, proof_pitch, a_chal, chal_pitch, a_u, a_res, a_gt, gt_pitch, n, nullptr};
-    if (in_ce) {
-      // rows 0..53 of the lane buffer belong to a prove call that may still be in flight on this lane: verify stages elsewhere
-      uint8_t *d_proof = base + 26 * C, *d_chal = base + 54 * C, *d_u = base + 59 * C;
-      CUDA_TRY(ctx, cudaMemcpy2DAsync(d_proof, C, proof, proof_pitch, n, 27, cudaMemcpyHostToDevice, st));
-      CUDA_TRY(ctx, cudaMemcpy2DAsync(d_chal, C, chal, chal_pitch, n, 5, cudaMemcpyHostToDevice, st));
-      CUDA_TRY(ctx, cudaMemcpyAsync(d_u, u, n, cudaMemcpyHostToDevice, st));
-      A.proof = d_proof; A.proof_pitch = C; A.chal = d_chal; A.chal_pitch = C; A.u = d_u;
-    }
-    if (out_ce) { A.result = base + 60 * C; if (gt) { A.gt = base; A.gt_pitch = C; } }
-    const int keep = ctx->grid_scale;
-    ctx->grid_scale = (in_ce && out_ce) ? 2 : 1;
-    rc = launch_verify(ctx, st, A);
-    ctx->grid_scale = keep;
-    if (rc) return rc;
-    if (out_ce) {
-      CUDA_TRY(ctx, cudaMemcpyAsync(result, A.result, n, cudaMemcpyDeviceToHost, st));
-      if (gt) CUDA_TRY(ctx, cudaMemcpy2DAsync(gt, gt_pitch, A.gt, C, n, 4, cudaMemcpyDeviceToHost, st));
-    }
-    return PBH_OK;
-  }
-  rc = pbh_ctx_sync(ctx);
-  if (rc) return rc;
-  return pbh_verify_batch(ctx, n, proof, proof_pitch, chal, chal_pitch, u, result, gt, gt_pitch);
+  const char* bad = !proof || !chal || !u || !result ? "null pointer"
+                    : proof_pitch < n || chal_pitch < n || (gt && gt_pitch < n) ? "pitch < n" : nullptr;
+  VerifyArgs A{proof, proof_pitch, chal, chal_pitch, u, result, gt, gt_pitch, n, nullptr};
+  bool stage_in = false, stage_out = false;
+  return lane_call(ctx, lane, n, bad,
+      [&] {
+        const VerifyArgs M = mapped(ctx, A);
+        const LanePlan p = plane_plan(ctx, n, VR::kRows, host_pinned(proof) && host_pinned(chal) && host_pinned(u), M.proof && M.chal && M.u,
+                                      host_pinned(result) && (!gt || host_pinned(gt)), M.result && (!gt || M.gt), &stage_in, &stage_out);
+        if (!stage_in) { A.proof = M.proof; A.chal = M.chal; A.u = M.u; }
+        if (!stage_out) { A.result = M.result; A.gt = M.gt; }
+        return p;
+      },
+      [&](cudaStream_t st, uint8_t* base, size_t C, const void*) { return verify_body(ctx, st, base, C, A, stage_in, stage_out); },
+      [&] { return pbh_verify_batch(ctx, n, proof, proof_pitch, chal, chal_pitch, u, result, gt, gt_pitch); });
 }
 int pbh_lane_sync(pbh_ctx* ctx, int lane) {
   CTX_CHECK(ctx);
   cudaStream_t st;
-  int rc = lane_stream(ctx, lane, &st);
-  if (rc) return rc;
+  PBH_TRY(lane_stream(ctx, lane, &st));
   ctx->resident_host[lane] = nullptr;   // after a sync the caller may change its buffers
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   CUDA_TRY(ctx, cudaStreamSynchronize(st));
@@ -1182,6 +1251,32 @@ int pbh_ctx_get_fs_seed(const pbh_ctx* ctx, uint8_t seed[32]) {
     for (int b = 0; b < 4; b++) seed[4 * i + b] = (uint8_t)(ctx->hs.fs_seed[i] >> (24 - 8 * b));
   return PBH_OK;
 }
+// The compile-time <ALGO, FP32, PBH_CIRCUIT> of the Fiat-Shamir provers for a context, handed to f as an FsProver<...>.  Five
+// instantiations: both algorithms with the FP32 or the int32 prover, and the TABLE FP32 prover for the reference's own circuit.
+template <int ALGO, bool FP32, bool PBH_CIRCUIT>
+struct FsProver {
+  static constexpr int algo = ALGO;
+  static constexpr bool fp32 = FP32, pbh_circuit = PBH_CIRCUIT;
+};
+template <class F>
+static void with_fs_prover(const pbh_ctx* ctx, F f) {
+  const bool special = ctx->pbh_circuit && ctx->specialise;
+  if (ctx->algo == PBH_ALGO_TABLE) {
+    if (!ctx->prover_fp32) f(FsProver<ALGO_TABLE, false, false>{});
+    else if (special) f(FsProver<ALGO_TABLE, true, true>{});
+    else f(FsProver<ALGO_TABLE, true, false>{});
+  } else {
+    if (!ctx->prover_fp32) f(FsProver<ALGO_ARITH, false, false>{});
+    else f(FsProver<ALGO_ARITH, true, false>{});
+  }
+}
+// The same for the Fiat-Shamir verifiers: <ALGO> as a std::integral_constant, and the run-time fp32 flag (TABLE only).
+template <class F>
+static void with_fs_verifier(const pbh_ctx* ctx, F f) {
+  if (ctx->algo == PBH_ALGO_TABLE) f(std::integral_constant<int, ALGO_TABLE>{}, ctx->verifier_fp32 != 0);
+  else f(std::integral_constant<int, ALGO_ARITH>{}, false);
+}
+
 // digest (nullable): device uint64, overwritten with the digest of the 27 proof planes (items first_index ..).  The FP32 provers
 // add it in the kernel (launch-local record, no memset); the int32 prover has no such instantiation and runs the digest kernel
 // on a zeroed word after it, as launch_prove does off the TMA path.
@@ -1189,30 +1284,26 @@ static int launch_prove_fs(pbh_ctx* ctx, cudaStream_t st, const ProveFsArgs& F, 
   if (F.base.n == 0) return PBH_OK;
   const int grid = grid_for(ctx, F.base.n, 2);
   const FsSeed seed = fs_seed_of(ctx);
-  const bool special = ctx->pbh_circuit && ctx->specialise;
-  if (digest && ctx->prover_fp32) {
+  const bool fused = digest && ctx->prover_fp32;
+  FsDigestArgs D{};
+  if (fused) {
     unsigned int* tc = fresh_tile_counter(ctx, st);
     if (!tc) return fail(ctx, PBH_ERR_UNSUPPORTED, "too many launches captured into CUDA graphs from this context");
-    const FsDigestArgs D{first_index, (unsigned long long*)digest, tc, peer_window_for(ctx, digest, sizeof(uint64_t))};
-    if (ctx->algo == PBH_ALGO_TABLE && special) prove_fs_kernel<ALGO_TABLE, true, true, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, D);
-    else if (ctx->algo == PBH_ALGO_TABLE) prove_fs_kernel<ALGO_TABLE, true, false, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, D);
-    else prove_fs_kernel<ALGO_ARITH, true, false, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, D);
-    ctx->launches++;
-    CUDA_TRY(ctx, cudaGetLastError());
-    return PBH_OK;
+    D = FsDigestArgs{first_index, (unsigned long long*)digest, tc, peer_window_for(ctx, digest, sizeof(uint64_t))};
   }
-  const FsDigestArgs none{};
-  if (ctx->algo == PBH_ALGO_TABLE) {
-    if (!ctx->prover_fp32) prove_fs_kernel<ALGO_TABLE, false, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, none);
-    else if (special) prove_fs_kernel<ALGO_TABLE, true, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, none);
-    else prove_fs_kernel<ALGO_TABLE, true, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, none);
-  } else {
-    if (!ctx->prover_fp32) prove_fs_kernel<ALGO_ARITH, false, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, none);
-    else prove_fs_kernel<ALGO_ARITH, true, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, none);
-  }
+  with_fs_prover(ctx, [&](auto P) {
+    using I = decltype(P);
+    if constexpr (I::fp32) {
+      if (fused) {
+        prove_fs_kernel<I::algo, true, I::pbh_circuit, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, D);
+        return;
+      }
+    }
+    prove_fs_kernel<I::algo, I::fp32, I::pbh_circuit><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, F, D);
+  });
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());
-  if (digest) {
+  if (digest && !fused) {
     CUDA_TRY(ctx, cudaMemsetAsync(digest, 0, sizeof(uint64_t), st));
     PBH_TRY(launch_digest(ctx, st, F.base.n, first_index, 27, F.base.proof, F.base.proof_pitch, digest));
     return launch_publish(ctx, st, digest, sizeof(uint64_t), peer_window_for(ctx, digest, sizeof(uint64_t)));
@@ -1228,13 +1319,10 @@ static int launch_verify_fs(pbh_ctx* ctx, cudaStream_t st, const VerifyFsArgs& F
   uint8_t* bitmap = F.base.bitmap;
   const PeerWindow pw = peer_window_for(ctx, bitmap, (F.base.n + 7) / 8);
   const bool fused = bitmap && ((uintptr_t)bitmap % 4) == 0;
-  if (fused) {
-    if (ctx->algo == PBH_ALGO_TABLE) verify_fs_kernel<ALGO_TABLE, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, ctx->verifier_fp32 != 0, seed, ctx->d_tables, F, pw);
-    else verify_fs_kernel<ALGO_ARITH, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, false, seed, ctx->d_tables, F, pw);
-  } else {
-    if (ctx->algo == PBH_ALGO_TABLE) verify_fs_kernel<ALGO_TABLE><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, ctx->verifier_fp32 != 0, seed, ctx->d_tables, F, PeerWindow{});
-    else verify_fs_kernel<ALGO_ARITH><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, false, seed, ctx->d_tables, F, PeerWindow{});
-  }
+  with_fs_verifier(ctx, [&](auto algo, bool fp32) {
+    if (fused) verify_fs_kernel<decltype(algo)::value, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, fp32, seed, ctx->d_tables, F, pw);
+    else verify_fs_kernel<decltype(algo)::value><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, fp32, seed, ctx->d_tables, F, PeerWindow{});
+  });
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());
   if (bitmap && !fused) {
@@ -1295,15 +1383,16 @@ int pbh_prove_fs_batch(pbh_ctx* ctx, size_t n, const uint8_t* wit, size_t wit_pi
   if (wit_pitch < n || rand_pitch < n || proof_pitch < n || (chal_out && chal_pitch < n)) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "pitch < n");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   return for_each_chunk(ctx, n, [&](size_t lo, size_t m, size_t C, uint8_t* base, cudaStream_t st) -> int {
-    uint8_t *d_wit = base, *d_rnd = base + 12 * C, *d_proof = base + 21 * C, *d_status = base + 48 * C, *d_chal = base + 49 * C;
-    PBH_TRY(stage_h2d(ctx, base, st, d_wit, C, wit + lo, wit_pitch, m, 12));
-    PBH_TRY(stage_h2d(ctx, base, st, d_rnd, C, rnd + lo, rand_pitch, m, 9));
+    uint8_t *d_wit = at_row(base, C, PR::wit), *d_rnd = at_row(base, C, PR::rnd), *d_proof = at_row(base, C, PR::proof),
+            *d_status = at_row(base, C, PR::status), *d_chal = at_row(base, C, FsRows::chal_out);
+    PBH_TRY(stage_h2d(ctx, base, st, d_wit, C, wit + lo, wit_pitch, m, PR::wit.count));
+    PBH_TRY(stage_h2d(ctx, base, st, d_rnd, C, rnd + lo, rand_pitch, m, PR::rnd.count));
     ProveFsArgs F{{d_wit, C, d_rnd, C, nullptr, 0, d_proof, C, d_status, m}, chal_out ? d_chal : nullptr, C};
     int rc = launch_prove_fs(ctx, st, F);
     if (rc) return rc;
-    PBH_TRY(stage_d2h(ctx, base, st, proof + lo, proof_pitch, d_proof, C, m, 27));
+    PBH_TRY(stage_d2h(ctx, base, st, proof + lo, proof_pitch, d_proof, C, m, PR::proof.count));
     PBH_TRY(stage_d2h(ctx, base, st, status + lo, 0, d_status, 0, m, 1));
-    if (chal_out) PBH_TRY(stage_d2h(ctx, base, st, chal_out + lo, chal_pitch, d_chal, C, m, 6));
+    if (chal_out) PBH_TRY(stage_d2h(ctx, base, st, chal_out + lo, chal_pitch, d_chal, C, m, FsRows::chal_out.count));
     return PBH_OK;
   });
 }
@@ -1315,14 +1404,15 @@ int pbh_verify_fs_batch(pbh_ctx* ctx, size_t n, const uint8_t* proof, size_t pro
   if (proof_pitch < n || (chal_out && chal_pitch < n) || (gt && gt_pitch < n)) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "pitch < n");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   return for_each_chunk(ctx, n, [&](size_t lo, size_t m, size_t C, uint8_t* base, cudaStream_t st) -> int {
-    uint8_t *d_proof = base, *d_res = base + 27 * C, *d_chal = base + 28 * C, *d_gt = base + 34 * C;
-    PBH_TRY(stage_h2d(ctx, base, st, d_proof, C, proof + lo, proof_pitch, m, 27));
+    uint8_t *d_proof = at_row(base, C, VR::proof), *d_res = at_row(base, C, VR::res), *d_chal = at_row(base, C, FsRows::chal_out),
+            *d_gt = at_row(base, C, VR::gt);
+    PBH_TRY(stage_h2d(ctx, base, st, d_proof, C, proof + lo, proof_pitch, m, VR::proof.count));
     VerifyFsArgs F{{d_proof, C, nullptr, 0, nullptr, d_res, gt ? d_gt : nullptr, C, m, nullptr}, chal_out ? d_chal : nullptr, C};
     int rc = launch_verify_fs(ctx, st, F);
     if (rc) return rc;
     PBH_TRY(stage_d2h(ctx, base, st, result + lo, 0, d_res, 0, m, 1));
-    if (chal_out) PBH_TRY(stage_d2h(ctx, base, st, chal_out + lo, chal_pitch, d_chal, C, m, 6));
-    if (gt) PBH_TRY(stage_d2h(ctx, base, st, gt + lo, gt_pitch, d_gt, C, m, 4));
+    if (chal_out) PBH_TRY(stage_d2h(ctx, base, st, chal_out + lo, chal_pitch, d_chal, C, m, FsRows::chal_out.count));
+    if (gt) PBH_TRY(stage_d2h(ctx, base, st, gt + lo, gt_pitch, d_gt, C, m, VR::gt.count));
     return PBH_OK;
   });
 }
@@ -1373,9 +1463,10 @@ int pbh_prove_records(pbh_ctx* ctx, size_t n, const pbh_witness_record* in, pbh_
   if (!in || !out) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   return for_each_chunk(ctx, n, [&](size_t lo, size_t m, size_t C, uint8_t* base, cudaStream_t st) -> int {
-    uint8_t *d_wit = base, *d_rnd = base + 12 * C, *d_chal = base + 21 * C, *d_proof = base + 26 * C, *d_status = base + 53 * C;
-    pbh_witness_record* d_in = reinterpret_cast<pbh_witness_record*>(base + 64 * C);
-    pbh_proof_record* d_out = reinterpret_cast<pbh_proof_record*>(base + 96 * C);
+    uint8_t *d_wit = at_row(base, C, PR::wit), *d_rnd = at_row(base, C, PR::rnd), *d_chal = at_row(base, C, PR::chal),
+            *d_proof = at_row(base, C, PR::proof), *d_status = at_row(base, C, PR::status);
+    pbh_witness_record* d_in = at_row<pbh_witness_record>(base, C, RecordRows::witness);
+    pbh_proof_record* d_out = at_row<pbh_proof_record>(base, C, RecordRows::proof);
     PBH_TRY(stage_h2d(ctx, base, st, d_in, 0, in + lo, 0, m * sizeof(pbh_witness_record), 1));
     witness_records_to_planes_kernel<<<grid_for(ctx, m, 8), kBlock, 0, st>>>(m, d_in, d_wit, C, d_rnd, C, d_chal, C, nullptr);
     ctx->launches++;
@@ -1396,19 +1487,15 @@ int pbh_verify_records(pbh_ctx* ctx, size_t n, const pbh_proof_record* proofs, c
   if (!proofs || !params || !result) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   return for_each_chunk(ctx, n, [&](size_t lo, size_t m, size_t C, uint8_t* base, cudaStream_t st) -> int {
-    uint8_t *d_proof = base, *d_chal = base + 27 * C, *d_u = base + 32 * C, *d_res = base + 33 * C;
-    pbh_witness_record* d_par = reinterpret_cast<pbh_witness_record*>(base + 64 * C);
-    pbh_proof_record* d_prf = reinterpret_cast<pbh_proof_record*>(base + 96 * C);
+    uint8_t *d_proof = at_row(base, C, VR::proof), *d_chal = at_row(base, C, VR::chal), *d_u = at_row(base, C, VR::u);
+    pbh_witness_record* d_par = at_row<pbh_witness_record>(base, C, RecordRows::witness);
+    pbh_proof_record* d_prf = at_row<pbh_proof_record>(base, C, RecordRows::proof);
     PBH_TRY(stage_h2d(ctx, base, st, d_prf, 0, proofs + lo, 0, m * sizeof(pbh_proof_record), 1));
     PBH_TRY(stage_h2d(ctx, base, st, d_par, 0, params + lo, 0, m * sizeof(pbh_witness_record), 1));
     proof_records_to_planes_kernel<<<grid_for(ctx, m, 8), kBlock, 0, st>>>(m, d_prf, d_proof, C, nullptr);
     witness_records_to_planes_kernel<<<grid_for(ctx, m, 8), kBlock, 0, st>>>(m, d_par, nullptr, 0, nullptr, 0, d_chal, C, d_u);
     ctx->launches += 2;
-    VerifyArgs A{d_proof, C, d_chal, C, d_u, d_res, nullptr, 0, m, nullptr};
-    int rc = launch_verify(ctx, st, A);
-    if (rc) return rc;
-    PBH_TRY(stage_d2h(ctx, base, st, result + lo, 0, d_res, 0, m, 1));
-    return PBH_OK;
+    return verify_body(ctx, st, base, C, VerifyArgs{d_proof, C, d_chal, C, d_u, result + lo, nullptr, 0, m, nullptr}, false, true);
   });
 }
 
@@ -1469,15 +1556,14 @@ int pbh_unpack_proof_dev(pbh_ctx* ctx, size_t n, const pbh_packed_proof* in, con
   return launch_unpack_proof(ctx, ctx->compute, n, in, chal_u, proof, proof_pitch, status, chal, chal_pitch, u);
 }
 
-// One chunk (or one whole lane batch) of the packed prover / verifier on stream st, staged in `base` (rows of C bytes):
-// planes below row 64 as in the byte-plane bodies, packed prover input in rows 64..79, packed proofs out in 80..91, the
-// verifier's packed proofs in 96..107 and its challenge words in 108..111.
+// One chunk (or one whole lane batch) of the packed prover / verifier on stream st, staged in `base` (PackedRows).
 static int packed_prove_body(pbh_ctx* ctx, cudaStream_t st, uint8_t* base, size_t C, size_t m, const pbh_packed_witness* in,
                              pbh_packed_proof* out, uint8_t* result_host) {
-  uint8_t *d_wit = base, *d_rnd = base + 12 * C, *d_chal = base + 21 * C, *d_proof = base + 26 * C, *d_status = base + 53 * C,
-          *d_u = base + 54 * C, *d_res = base + 55 * C;
-  pbh_packed_witness* d_in = reinterpret_cast<pbh_packed_witness*>(base + 64 * C);
-  pbh_packed_proof* d_out = reinterpret_cast<pbh_packed_proof*>(base + 80 * C);
+  uint8_t *d_wit = at_row(base, C, PR::wit), *d_rnd = at_row(base, C, PR::rnd), *d_chal = at_row(base, C, PR::chal),
+          *d_proof = at_row(base, C, PR::proof), *d_status = at_row(base, C, PR::status), *d_u = at_row(base, C, PR::u),
+          *d_res = at_row(base, C, PR::res);
+  pbh_packed_witness* d_in = at_row<pbh_packed_witness>(base, C, PackedRows::in);
+  pbh_packed_proof* d_out = at_row<pbh_packed_proof>(base, C, PackedRows::out);
   PBH_TRY(stage_h2d(ctx, base, st, d_in, 0, in, 0, m * sizeof(pbh_packed_witness), 1));
   int rc = launch_unpack_witness(ctx, st, m, d_in, d_wit, C, d_rnd, C, d_chal, C, result_host ? d_u : nullptr);
   if (rc) return rc;
@@ -1495,23 +1581,18 @@ static int packed_prove_body(pbh_ctx* ctx, cudaStream_t st, uint8_t* base, size_
   if (result_host) PBH_TRY(stage_d2h(ctx, base, st, result_host, 0, d_res, 0, m, 1));
   return PBH_OK;
 }
-// `resident`: the proof planes these packed proofs decode to are already at rows 26..52 of `base` - the prove call that produced
+// `resident`: the proof planes these packed proofs decode to are already at rows VR::proof of `base` - the prove call that produced
 // `proofs` on this lane left them there (packed_prove_body), and pack -> unpack is the identity on a prover's output - so neither
 // the upload of the proofs nor their decoding is repeated; only the challenge words travel.
 static int packed_verify_body(pbh_ctx* ctx, cudaStream_t st, uint8_t* base, size_t C, size_t m, const pbh_packed_proof* proofs,
                               const uint32_t* chal_u, uint8_t* result, bool resident = false) {
-  uint8_t *d_proof = base + 26 * C, *d_chal = base + 54 * C, *d_u = base + 59 * C, *d_res = base + 60 * C;
-  pbh_packed_proof* d_prf = reinterpret_cast<pbh_packed_proof*>(base + 96 * C);
-  uint32_t* d_cu = reinterpret_cast<uint32_t*>(base + 108 * C);
+  uint8_t *d_proof = at_row(base, C, VR::proof), *d_chal = at_row(base, C, VR::chal), *d_u = at_row(base, C, VR::u);
+  pbh_packed_proof* d_prf = at_row<pbh_packed_proof>(base, C, PackedRows::proofs);
+  uint32_t* d_cu = at_row<uint32_t>(base, C, PackedRows::chal_u);
   if (!resident) PBH_TRY(stage_h2d(ctx, base, st, d_prf, 0, proofs, 0, m * sizeof(pbh_packed_proof), 1));
   PBH_TRY(stage_h2d(ctx, base, st, d_cu, 0, chal_u, 0, m * sizeof(uint32_t), 1));
-  int rc = launch_unpack_proof(ctx, st, m, resident ? nullptr : d_prf, d_cu, d_proof, C, nullptr, d_chal, C, d_u);
-  if (rc) return rc;
-  VerifyArgs A{d_proof, C, d_chal, C, d_u, d_res, nullptr, 0, m, nullptr};
-  rc = launch_verify(ctx, st, A);
-  if (rc) return rc;
-  PBH_TRY(stage_d2h(ctx, base, st, result, 0, d_res, 0, m, 1));
-  return PBH_OK;
+  PBH_TRY(launch_unpack_proof(ctx, st, m, resident ? nullptr : d_prf, d_cu, d_proof, C, nullptr, d_chal, C, d_u));
+  return verify_body(ctx, st, base, C, VerifyArgs{d_proof, C, d_chal, C, d_u, result, nullptr, 0, m, nullptr}, false, true);
 }
 
 int pbh_prove_packed(pbh_ctx* ctx, size_t n, const pbh_packed_witness* in, pbh_packed_proof* out) {
@@ -1543,67 +1624,31 @@ int pbh_verify_packed(pbh_ctx* ctx, size_t n, const pbh_packed_proof* proofs, co
 }
 int pbh_prove_packed_async(pbh_ctx* ctx, int lane, size_t n, const pbh_packed_witness* in, pbh_packed_proof* out) {
   CTX_CHECK(ctx);
-  cudaStream_t st;
-  int rc = lane_stream(ctx, lane, &st);
-  if (rc) return rc;
-  ctx->resident_host[lane] = nullptr;
-  if (n == 0) return PBH_OK;
-  if (!in || !out) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
-  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  if (n <= kLaneMaxItems && host_pinned(reinterpret_cast<const uint8_t*>(in)) && host_pinned(reinterpret_cast<const uint8_t*>(out))) {
-    const size_t C = (n + kTile - 1) / kTile * kTile;
-    rc = ensure_lane(ctx, lane, kStagePlanes * C);
-    if (rc) return rc;
-    rc = packed_prove_body(ctx, st, ctx->lane_buf[lane], C, n, in, out, nullptr);
-    if (rc == PBH_OK && ctx->proof_resident) { ctx->resident_host[lane] = out; ctx->resident_n[lane] = n; }
-    return rc;
-  }
-  rc = pbh_ctx_sync(ctx);
-  if (rc) return rc;
-  return pbh_prove_packed(ctx, n, in, out);
+  return lane_call(ctx, lane, n, !in || !out ? "null pointer" : nullptr, [&] { return staged_plan(n, PackedRows::kProveRows, {in, out}); },
+      [&](cudaStream_t st, uint8_t* base, size_t C, const void*) -> int {
+        PBH_TRY(packed_prove_body(ctx, st, base, C, n, in, out, nullptr));
+        if (ctx->proof_resident) { ctx->resident_host[lane] = out; ctx->resident_n[lane] = n; }
+        return PBH_OK;
+      },
+      [&] { return pbh_prove_packed(ctx, n, in, out); });
 }
 int pbh_prove_verify_packed_async(pbh_ctx* ctx, int lane, size_t n, const pbh_packed_witness* in, pbh_packed_proof* out, uint8_t* result) {
   CTX_CHECK(ctx);
-  cudaStream_t st;
-  int rc = lane_stream(ctx, lane, &st);
-  if (rc) return rc;
-  ctx->resident_host[lane] = nullptr;
-  if (n == 0) return PBH_OK;
-  if (!in || !out || !result) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
-  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  if (n <= kLaneMaxItems && host_pinned(reinterpret_cast<const uint8_t*>(in)) && host_pinned(reinterpret_cast<const uint8_t*>(out)) && host_pinned(result)) {
-    const size_t C = (n + kTile - 1) / kTile * kTile;
-    rc = ensure_lane(ctx, lane, kStagePlanes * C);
-    if (rc) return rc;
-    return packed_prove_body(ctx, st, ctx->lane_buf[lane], C, n, in, out, result);
-  }
-  rc = pbh_ctx_sync(ctx);
-  if (rc) return rc;
-  return pbh_prove_verify_packed(ctx, n, in, out, result);
+  return lane_call(ctx, lane, n, !in || !out || !result ? "null pointer" : nullptr,
+      [&] { return staged_plan(n, PackedRows::kProveRows, {in, out, result}); },
+      [&](cudaStream_t st, uint8_t* base, size_t C, const void*) { return packed_prove_body(ctx, st, base, C, n, in, out, result); },
+      [&] { return pbh_prove_verify_packed(ctx, n, in, out, result); });
 }
 int pbh_verify_packed_async(pbh_ctx* ctx, int lane, size_t n, const pbh_packed_proof* proofs, const uint32_t* chal_u, uint8_t* result) {
   CTX_CHECK(ctx);
-  cudaStream_t st;
-  int rc = lane_stream(ctx, lane, &st);
-  if (rc) return rc;
-  size_t res_n = 0;
-  const void* res_host = take_resident(ctx, lane, &res_n);
-  if (n == 0) return PBH_OK;
-  if (!proofs || !chal_u || !result) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
-  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  if (n <= kLaneMaxItems && host_pinned(reinterpret_cast<const uint8_t*>(proofs)) && host_pinned(reinterpret_cast<const uint8_t*>(chal_u)) &&
-      host_pinned(result)) {
-    const size_t C = (n + kTile - 1) / kTile * kTile;
-    rc = ensure_lane(ctx, lane, kStagePlanes * C);
-    if (rc) return rc;
-    // the very buffer the previous call on this lane is still filling, with no synchronisation in between (the caller may not
-    // touch it before pbh_lane_sync): its contents ARE the proofs resident in the lane buffer
-    const bool resident = ctx->proof_resident && res_host == static_cast<const void*>(proofs) && res_n == n;
-    return packed_verify_body(ctx, st, ctx->lane_buf[lane], C, n, proofs, chal_u, result, resident);
-  }
-  rc = pbh_ctx_sync(ctx);
-  if (rc) return rc;
-  return pbh_verify_packed(ctx, n, proofs, chal_u, result);
+  return lane_call(ctx, lane, n, !proofs || !chal_u || !result ? "null pointer" : nullptr,
+      [&] { return staged_plan(n, PackedRows::kVerifyRows, {proofs, chal_u, result}); },
+      [&](cudaStream_t st, uint8_t* base, size_t C, const void* resident) {
+        // the very buffer the previous call on this lane is still filling, with no synchronisation in between (the caller may not
+        // touch it before pbh_lane_sync): its contents ARE the proofs resident in the lane buffer
+        return packed_verify_body(ctx, st, base, C, n, proofs, chal_u, result, ctx->proof_resident && resident == proofs);
+      },
+      [&] { return pbh_verify_packed(ctx, n, proofs, chal_u, result); });
 }
 
 // host-side format conversion: the codec of pbh_packed.cuh on the CPU (no context, no device)
@@ -1680,17 +1725,12 @@ static int launch_prove_fs_packed(pbh_ctx* ctx, cudaStream_t st, size_t n, const
   if (n == 0) return PBH_OK;
   const int grid = grid_for(ctx, n, 2);
   const FsSeed seed = fs_seed_of(ctx);
-  const bool special = ctx->pbh_circuit && ctx->specialise;
   const uint32_t* i32 = reinterpret_cast<const uint32_t*>(in);
   uint32_t* o32 = reinterpret_cast<uint32_t*>(out);
-  if (ctx->algo == PBH_ALGO_TABLE) {
-    if (!ctx->prover_fp32) prove_fs_packed_kernel<ALGO_TABLE, false, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, n, i32, o32, chal_u_out);
-    else if (special) prove_fs_packed_kernel<ALGO_TABLE, true, true><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, n, i32, o32, chal_u_out);
-    else prove_fs_packed_kernel<ALGO_TABLE, true, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, n, i32, o32, chal_u_out);
-  } else {
-    if (!ctx->prover_fp32) prove_fs_packed_kernel<ALGO_ARITH, false, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, n, i32, o32, chal_u_out);
-    else prove_fs_packed_kernel<ALGO_ARITH, true, false><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, n, i32, o32, chal_u_out);
-  }
+  with_fs_prover(ctx, [&](auto P) {
+    using I = decltype(P);
+    prove_fs_packed_kernel<I::algo, I::fp32, I::pbh_circuit><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, seed, ctx->d_tables, n, i32, o32, chal_u_out);
+  });
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());
   return PBH_OK;
@@ -1700,9 +1740,9 @@ static int launch_verify_fs_packed(pbh_ctx* ctx, cudaStream_t st, size_t n, cons
   const int grid = grid_for(ctx, n, 2);
   const FsSeed seed = fs_seed_of(ctx);
   const uint32_t* p32 = reinterpret_cast<const uint32_t*>(proofs);
-  if (ctx->algo == PBH_ALGO_TABLE)
-    verify_fs_packed_kernel<ALGO_TABLE><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, ctx->verifier_fp32 != 0, seed, ctx->d_tables, n, p32, result);
-  else verify_fs_packed_kernel<ALGO_ARITH><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, false, seed, ctx->d_tables, n, p32, result);
+  with_fs_verifier(ctx, [&](auto algo, bool fp32) {
+    verify_fs_packed_kernel<decltype(algo)::value><<<grid, 256, 0, st>>>(ctx->hs.K, ctx->hs.KF, fp32, seed, ctx->d_tables, n, p32, result);
+  });
   ctx->launches++;
   CUDA_TRY(ctx, cudaGetLastError());
   return PBH_OK;
@@ -1726,16 +1766,12 @@ int pbh_verify_fs_packed_dev(pbh_ctx* ctx, size_t n, const pbh_packed_proof* pro
   return launch_verify_fs_packed(ctx, ctx->compute, n, proofs, result);
 }
 
-// One chunk (or one whole lane batch) on stream st, staged in `base` (rows of C bytes): the prover's records in rows 64..75, its
-// proofs in 80..91 and challenge words in 92..95; the verifier's proofs in 96..107 and results in row 108.  Prover and verifier
-// rows are disjoint, so a verify enqueued on a lane behind a prove never overwrites rows that prove still has to download.
-static_assert(64 + sizeof(pbh_packed_fs_witness) <= 80 && 80 + sizeof(pbh_packed_proof) + 4 <= 96 && 96 + sizeof(pbh_packed_proof) + 1 <= kStagePlanes,
-              "packed Fiat-Shamir bodies: prover rows 64..95, verifier rows 96..108");
+// One chunk (or one whole lane batch) on stream st, staged in `base` (FsPackedRows).
 static int fs_packed_prove_body(pbh_ctx* ctx, cudaStream_t st, uint8_t* base, size_t C, size_t m, const pbh_packed_fs_witness* in,
                                 pbh_packed_proof* out, uint32_t* chal_u_out) {
-  pbh_packed_fs_witness* d_in = reinterpret_cast<pbh_packed_fs_witness*>(base + 64 * C);
-  pbh_packed_proof* d_out = reinterpret_cast<pbh_packed_proof*>(base + 80 * C);
-  uint32_t* d_cu = reinterpret_cast<uint32_t*>(base + 92 * C);
+  pbh_packed_fs_witness* d_in = at_row<pbh_packed_fs_witness>(base, C, FsPackedRows::in);
+  pbh_packed_proof* d_out = at_row<pbh_packed_proof>(base, C, FsPackedRows::out);
+  uint32_t* d_cu = at_row<uint32_t>(base, C, FsPackedRows::chal_u);
   PBH_TRY(stage_h2d(ctx, base, st, d_in, 0, in, 0, m * sizeof(pbh_packed_fs_witness), 1));
   PBH_TRY(launch_prove_fs_packed(ctx, st, m, d_in, d_out, chal_u_out ? d_cu : nullptr));
   PBH_TRY(stage_d2h(ctx, base, st, out, 0, d_out, 0, m * sizeof(pbh_packed_proof), 1));
@@ -1744,8 +1780,8 @@ static int fs_packed_prove_body(pbh_ctx* ctx, cudaStream_t st, uint8_t* base, si
 }
 static int fs_packed_verify_body(pbh_ctx* ctx, cudaStream_t st, uint8_t* base, size_t C, size_t m, const pbh_packed_proof* proofs,
                                  uint8_t* result) {
-  pbh_packed_proof* d_prf = reinterpret_cast<pbh_packed_proof*>(base + 96 * C);
-  uint8_t* d_res = base + 108 * C;
+  pbh_packed_proof* d_prf = at_row<pbh_packed_proof>(base, C, FsPackedRows::proofs);
+  uint8_t* d_res = at_row(base, C, FsPackedRows::res);
   PBH_TRY(stage_h2d(ctx, base, st, d_prf, 0, proofs, 0, m * sizeof(pbh_packed_proof), 1));
   PBH_TRY(launch_verify_fs_packed(ctx, st, m, d_prf, d_res));
   PBH_TRY(stage_d2h(ctx, base, st, result, 0, d_res, 0, m, 1));
@@ -1770,55 +1806,18 @@ int pbh_verify_fs_packed(pbh_ctx* ctx, size_t n, const pbh_packed_proof* proofs,
     return fs_packed_verify_body(ctx, st, base, C, m, proofs + lo, result + lo);
   });
 }
-// A lane call that fails after enqueueing copies waits for them: the caller may release its buffers once the call has returned.
-static int lane_settle(pbh_ctx* ctx, cudaStream_t st, int rc) {
-  if (rc != PBH_OK) {
-    const std::string keep = ctx->last_error;
-    cudaStreamSynchronize(st);
-    cudaGetLastError();
-    ctx->last_error = keep;
-  }
-  return rc;
-}
 int pbh_prove_fs_packed_async(pbh_ctx* ctx, int lane, size_t n, const pbh_packed_fs_witness* in, pbh_packed_proof* out, uint32_t* chal_u_out) {
   CTX_CHECK(ctx);
-  cudaStream_t st;
-  int rc = lane_stream(ctx, lane, &st);
-  if (rc) return rc;
-  ctx->resident_host[lane] = nullptr;
-  if (n == 0) return PBH_OK;
-  if (!in || !out) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
-  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  if (n <= kLaneMaxItems && host_pinned(reinterpret_cast<const uint8_t*>(in)) && host_pinned(reinterpret_cast<const uint8_t*>(out)) &&
-      (!chal_u_out || host_pinned(reinterpret_cast<const uint8_t*>(chal_u_out)))) {
-    const size_t C = (n + kTile - 1) / kTile * kTile;
-    rc = ensure_lane(ctx, lane, kStagePlanes * C);
-    if (rc) return rc;
-    return lane_settle(ctx, st, fs_packed_prove_body(ctx, st, ctx->lane_buf[lane], C, n, in, out, chal_u_out));
-  }
-  rc = pbh_ctx_sync(ctx);
-  if (rc) return rc;
-  return pbh_prove_fs_packed(ctx, n, in, out, chal_u_out);
+  return lane_call(ctx, lane, n, !in || !out ? "null pointer" : nullptr, [&] { return staged_plan(n, FsPackedRows::kProveRows, {in, out, chal_u_out}); },
+      [&](cudaStream_t st, uint8_t* base, size_t C, const void*) { return fs_packed_prove_body(ctx, st, base, C, n, in, out, chal_u_out); },
+      [&] { return pbh_prove_fs_packed(ctx, n, in, out, chal_u_out); });
 }
 // No resident-proof shortcut here (PBH_OPT_PROOF_RESIDENT): the verifier uploads the buffer it is handed, whatever ran before.
 int pbh_verify_fs_packed_async(pbh_ctx* ctx, int lane, size_t n, const pbh_packed_proof* proofs, uint8_t* result) {
   CTX_CHECK(ctx);
-  cudaStream_t st;
-  int rc = lane_stream(ctx, lane, &st);
-  if (rc) return rc;
-  ctx->resident_host[lane] = nullptr;
-  if (n == 0) return PBH_OK;
-  if (!proofs || !result) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
-  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  if (n <= kLaneMaxItems && host_pinned(reinterpret_cast<const uint8_t*>(proofs)) && host_pinned(result)) {
-    const size_t C = (n + kTile - 1) / kTile * kTile;
-    rc = ensure_lane(ctx, lane, kStagePlanes * C);
-    if (rc) return rc;
-    return lane_settle(ctx, st, fs_packed_verify_body(ctx, st, ctx->lane_buf[lane], C, n, proofs, result));
-  }
-  rc = pbh_ctx_sync(ctx);
-  if (rc) return rc;
-  return pbh_verify_fs_packed(ctx, n, proofs, result);
+  return lane_call(ctx, lane, n, !proofs || !result ? "null pointer" : nullptr, [&] { return staged_plan(n, FsPackedRows::kVerifyRows, {proofs, result}); },
+      [&](cudaStream_t st, uint8_t* base, size_t C, const void*) { return fs_packed_verify_body(ctx, st, base, C, n, proofs, result); },
+      [&] { return pbh_verify_fs_packed(ctx, n, proofs, result); });
 }
 
 int pbh_pack_fs_witness_host(size_t n, const uint8_t* wit, size_t wit_pitch, const uint8_t* rnd, size_t rand_pitch, pbh_packed_fs_witness* out) {
