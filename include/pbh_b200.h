@@ -418,7 +418,10 @@ int pbh_coset_ntt4_batch(pbh_ctx* ctx, size_t n, uint32_t k, const uint8_t* coef
 int pbh_coset_intt4_batch(pbh_ctx* ctx, size_t n, uint32_t k, const uint8_t* evals, size_t in_pitch, uint8_t* coeffs,
                           size_t out_pitch, int on_device);
 /* generic power-of-two NTT / iNTT over F_modulus (modulus < 2^16, size in {2,4,...,64}), values as
- * uint16 planes; reproduces CooleyTurkey::fft / fft_inv (src/fft.rs:66-78) for full-length input. */
+ * uint16 planes; reproduces CooleyTurkey::fft / fft_inv (src/fft.rs:66-78) for full-length input.  Inputs are reduced
+ * mod modulus first; omega need not be primitive.  Only the inverse needs size^-1 mod modulus (fft_inv): without one it
+ * returns PBH_ERR_SETUP_PANIC, as the reference's `inv().unwrap()` panics, while the forward transform computes (modulus 2,
+ * even moduli). */
 int pbh_ntt_generic_batch(pbh_ctx* ctx, size_t n, uint32_t modulus, uint32_t omega, uint32_t size, int inverse,
                           const uint16_t* in, size_t in_pitch_elems, uint16_t* out, size_t out_pitch_elems,
                           int on_device);
@@ -586,6 +589,12 @@ int pbh_multi_prove_verify_fs_sharded(pbh_multi* m, uint64_t n_total, uint64_t f
 /* ---- synthetic inputs (SURVEY.md §8d), device pointers ------------------------------------------ */
 #define PBH_DIST_UNIFORM 0   /* attempt k = 0 only: exercises every status class                    */
 #define PBH_DIST_FULLPATH 1  /* smallest k whose prove succeeds and whose verify reaches the pairing */
+/* The full-path search tries attempts k = 0 .. PBH_GEN_MAX_ATTEMPTS - 1.  An item none of them satisfies (a short SRS
+ * where every proof ends in PBH_ST_SRS_OOB or commits to the identity) gets attempt 0's draw with attempt byte 255.  On
+ * the reference's circuit and SRS an attempt succeeds with probability about 1/19, so the cap is never reached there.  Witnesses are drawn
+ * from the 289 solutions (x, y, z) of x^2 + y^2 = z^2 (wit = x y z x^2, x y z y^2, x^2 y^2 z^2 z^2); on a context whose
+ * gates and copy constraints no such row satisfies, PBH_DIST_FULLPATH returns PBH_ERR_UNSUPPORTED before any launch. */
+#define PBH_GEN_MAX_ATTEMPTS 4096
 /* Item i of the batch has global index first_index + i; its bytes depend only on (seed, global
  * index, dist), so any sharding generates the same batch.  Fills wit/rand/chal/u; `attempt`
  * (nullable, n bytes) receives the accepted k (saturating at 255). */

@@ -155,6 +155,7 @@ inline uint32_t draw(uint64_t base, uint32_t j, uint32_t range) {
   uint64_t r = splitmix64(base + (uint64_t)j * 0xD1B54A32D192ED03ull);
   return (uint32_t)(((unsigned __int128)r * range) >> 64);
 }
+constexpr uint32_t kGenMaxAttempts = 4096;   // PBH_GEN_MAX_ATTEMPTS of include/pbh_b200.h
 struct WitnessTable { uint8_t xyz[289][3]; };
 const WitnessTable& witness_table() {
   static WitnessTable t = [] {
@@ -758,8 +759,9 @@ int oracle_generate_inputs(const void* circuit, uint8_t s, uint32_t srs_n, uint8
       uint8_t w[12], r[9], c[5], uu = 0;
       uint32_t k = 0;
       for (;; k++) {
-        sample_attempt(seed, first_index + i, k, w, r, c, uu);
-        if (dist == 0) break;
+        // past PBH_GEN_MAX_ATTEMPTS (include/pbh_b200.h): attempt 0's draw, reported as attempt 255
+        sample_attempt(seed, first_index + i, k < kGenMaxAttempts ? k : 0, w, r, c, uu);
+        if (dist == 0 || k == kGenMaxAttempts) break;
         Proof pr;
         if (prove_one(*st, w, r, c, pr) != 0) continue;
         const G1P* pts[9] = {&pr.a_s, &pr.b_s, &pr.c_s, &pr.z_s, &pr.t_lo_s, &pr.t_mid_s, &pr.t_hi_s, &pr.w_z_s, &pr.w_z_omega_s};

@@ -1934,7 +1934,9 @@ int pbh_ntt_generic_batch(pbh_ctx* ctx, size_t n, uint32_t modulus, uint32_t ome
   for (uint32_t i = 0; i < size; i++) { tw[i] = (uint16_t)m; m = (uint32_t)(((uint64_t)m * (omega % modulus)) % modulus); }
   uint64_t len_inv = 1, b = size % modulus, e = modulus - 2;
   while (e) { if (e & 1) len_inv = len_inv * b % modulus; b = b * b % modulus; e >>= 1; }
-  if ((len_inv * (size % modulus)) % modulus != 1) return fail(ctx, PBH_ERR_SETUP_PANIC, "size has no inverse modulo the modulus (F::from(len).inv().unwrap() panics)");
+  // only fft_inv asks for the length inverse (src/fft.rs:72-78): the forward transform exists for every modulus
+  if (inverse && (len_inv * (size % modulus)) % modulus != 1)
+    return fail(ctx, PBH_ERR_SETUP_PANIC, "size has no inverse modulo the modulus (F::from(len).inv().unwrap() panics)");
   uint16_t* d_tw = stg.in(tw, 64, 64, 1, ce); CUDA_TRY(ctx, ce);
   const uint16_t* d_in = in; uint16_t* d_out = out; size_t ip = in_pitch, op = out_pitch;
   if (!on_device) {
@@ -2220,6 +2222,20 @@ int pbh_digest_dev(pbh_ctx* ctx, size_t n, uint64_t first_index, uint32_t planes
   return launch_digest(ctx, ctx->compute, n, first_index, planes, data, pitch, out);
 }
 
+// Whether some row of the generator's witness table (x^2 + y^2 = z^2, laid out as generate_kernel lays it out) satisfies the
+// context's gates and copy constraints.  Without one every full-path attempt ends in PBH_ST_UNSATISFIED.
+static bool fullpath_satisfiable(const Consts& K) {
+  for (uint32_t x = 0; x < 17; x++)
+    for (uint32_t y = 0; y < 17; y++)
+      for (uint32_t z = 0; z < 17; z++) {
+        if ((x * x + y * y) % 17 != (z * z) % 17) continue;
+        const uint32_t xx = x * x % 17, yy = y * y % 17, zz = z * z % 17;
+        const uint32_t w[12] = {x, y, z, xx, x, y, z, yy, xx, yy, zz, zz};
+        if (!unsatisfied(w, K)) return true;
+      }
+  return false;
+}
+
 int pbh_generate_inputs_dev(pbh_ctx* ctx, size_t n, uint64_t first_index, uint64_t seed, int dist, uint8_t* wit, size_t wit_pitch,
                             uint8_t* rnd, size_t rand_pitch, uint8_t* chal, size_t chal_pitch, uint8_t* u, uint8_t* attempt) {
   CTX_CHECK(ctx);
@@ -2227,6 +2243,8 @@ int pbh_generate_inputs_dev(pbh_ctx* ctx, size_t n, uint64_t first_index, uint64
   if (!wit || !rnd || !chal || !u) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "null pointer");
   if (wit_pitch < n || rand_pitch < n || chal_pitch < n) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "pitch < n");
   if (dist != PBH_DIST_UNIFORM && dist != PBH_DIST_FULLPATH) return fail(ctx, PBH_ERR_BAD_ARGUMENT, "unknown distribution");
+  if (dist == PBH_DIST_FULLPATH && !fullpath_satisfiable(ctx->hs.K))
+    return fail(ctx, PBH_ERR_UNSUPPORTED, "no witness of the generator's table satisfies this circuit: PBH_DIST_FULLPATH cannot succeed");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   GenArgs A{n, first_index, seed, dist, wit, wit_pitch, rnd, rand_pitch, chal, chal_pitch, u, attempt, ctx->d_wtab};
   generate_kernel<<<grid_for(ctx, n, 8), kBlock, 0, ctx->compute>>>(ctx->hs.K, ctx->d_tables, A);

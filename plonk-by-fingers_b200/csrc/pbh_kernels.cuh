@@ -1536,7 +1536,9 @@ __global__ void __launch_bounds__(kBlock) generate_kernel(const Consts K, const 
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < A.n; i += (size_t)gridDim.x * blockDim.x) {
     uint32_t w[12], r[9], c[5], uu = 0, k = 0;
     for (;; k++) {
-      uint64_t base = splitmix64(A.seed ^ ((A.first_index + i) * 0x9E3779B97F4A7C15ull) ^ ((uint64_t)k * 0xC2B2AE3D27D4EB4Full));
+      // past PBH_GEN_MAX_ATTEMPTS: attempt 0's draw, reported as attempt 255
+      const uint64_t kk = k < PBH_GEN_MAX_ATTEMPTS ? k : 0u;
+      uint64_t base = splitmix64(A.seed ^ ((A.first_index + i) * 0x9E3779B97F4A7C15ull) ^ (kk * 0xC2B2AE3D27D4EB4Full));
       const uint8_t* s = A.wtab + 3 * gen_draw(base, 0, 289);
       uint32_t x = s[0], y = s[1], z = s[2];
       uint32_t xx = mod17(x * x), yy = mod17(y * y), zz = mod17(z * z);
@@ -1546,7 +1548,7 @@ __global__ void __launch_bounds__(kBlock) generate_kernel(const Consts K, const 
 #pragma unroll
       for (int j = 0; j < 5; j++) c[j] = gen_draw(base, 10 + j, 17);
       uu = gen_draw(base, 15, 17);
-      if (A.dist == PBH_DIST_UNIFORM) break;
+      if (A.dist == PBH_DIST_UNIFORM || k == PBH_GEN_MAX_ATTEMPTS) break;
       ProofRegs P;
       uint32_t status = prove_one<ALGO_TABLE>(w, r, c, K, sT, P);
       if (status != 0u) continue;

@@ -98,8 +98,9 @@ INSTANTIATIONS = [
 ]
 
 # Kernels whose paths other test files compare with the oracle: the F_17 / curve / GT sweeps (test_sweep_paths.py,
-# test_gpu_parity.py, test_gpu_round2.py), the record and packed codecs (test_gpu_parity.py, test_packed_format.py) and the
-# seeded input generator (test_gpu_parity.py, smoke()).
+# test_gpu_parity.py, test_gpu_round2.py), the packed codecs (test_packed_format.py), and - at their path and context
+# edges, with a launch census - the input generator, the generic NTT and NTT product, the polynomial product, the KZG
+# commitment, the general division, the ragged add / subtract and the record transposes (test_sweep_kernel_edges.py).
 SWEEP_KERNELS = sorted(
     [f"ntt4_kernel<{i},{k}>" for i in (0, 1) for k in (1, 2, 3)]
     + [f"poly_mul_vec_kernel<{a},{b}>" for a in (2, 4, 6, 8) for b in (2, 4, 6, 8)]
